@@ -3,7 +3,7 @@
 the trace loop on BASELINE configs[1]: the Cornell-box-style scene ("cornell"), 1024x1024, diffuse+glossy DDFs,
 split schedule 16/8/4/2, depth 4, 1024 spp for the whole job.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A *step* is one call of the hot path over one batch: `--passes-per-step` passes (default 8) of the full 1024x1024
 frame = 8.4 M camera paths. The default K = 128 steps is the whole 1024-spp job. N GPUs: one process per GPU
@@ -13,6 +13,12 @@ collective is the all-reduce of the accumulators (sum, sumsq, count) at the end 
 Printed JSON keys are described in DESIGN.md §Measurement. `--impl reference` times the reference's own CPU
 implementation (oracle/_ref, the unmodified dimalit/ipt sources + the C2 plug-in; else the oracle port) on all host
 cores with forked single-threaded workers (drand48 is process-global, SURVEY.md §6).
+
+`--dump-outputs DIR` writes, after the timed steps, the accumulators the timed path leaves in its plane after its last
+step (what `ipt_plane_download` hands a caller) as DIR/sum.npy, DIR/sumsq.npy and DIR/count.npy (float32, H x W;
+merged over the ranks for N > 1). The seed and the pass ranges depend only on the arguments, so two builds run with the
+same arguments can be compared output for output. Frames above DUMP_LIMIT_BYTES are written as a fixed, seeded sample of
+pixels (the same for all three arrays), with the sampled flat pixel indices in DIR/pixel_index.npy (float64).
 """
 from __future__ import annotations
 
@@ -362,6 +368,7 @@ def measure(D, w, steps, warmup, pps, args, ranks_active=None, e2e_steps=0):
     if active and D.rank == 0:
         s_, q_, c_ = plane.download()
         out["image_mean"] = float(s_.sum(dtype=np.float64) / max(int(c_.sum(dtype=np.uint64)), 1))
+        out["accumulators"] = {"sum": s_, "sumsq": q_, "count": c_}
 
     # ---- end to end through the C ABI with HOST buffers --------------------------------------------------------------
     if e2e_steps:
@@ -492,6 +499,25 @@ def source_sha16():
     return h.hexdigest()[:16]
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(directory, accumulators):
+    """The plane's accumulators as float32 .npy files; a seeded pixel sample when the whole frame exceeds the limit."""
+    out = Path(directory)
+    out.mkdir(parents=True, exist_ok=True)
+    arrays = {k: np.asarray(v, np.float32) for k, v in accumulators.items()}
+    n = next(iter(arrays.values())).size
+    per_pixel = sum(a.itemsize for a in arrays.values())
+    if n * per_pixel > DUMP_LIMIT_BYTES:
+        k = (DUMP_LIMIT_BYTES - 4096) // (per_pixel + 8)  # 8 B per sampled index; 4 KB for the .npy headers
+        idx = np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
+        arrays = {name: a.reshape(-1)[idx] for name, a in arrays.items()}
+        arrays["pixel_index"] = idx.astype(np.float64)
+    for name, a in arrays.items():
+        np.save(out / f"{name}.npy", a)
+
+
 def run_ours(args):
     from ipt_b200 import build, capi
 
@@ -502,6 +528,8 @@ def run_ours(args):
     pps = args.passes_per_step
     e2e_steps = max(1, min(args.steps, args.e2e_steps))
     m = measure(D, w, args.steps, args.warmup, pps, args, e2e_steps=e2e_steps)
+    if args.dump_outputs and D.rank == 0:
+        dump_outputs(args.dump_outputs, m["accumulators"])
     elapsed = m["elapsed"]
     line = None
     if D.rank == 0:
@@ -568,7 +596,7 @@ def run_ours(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=128)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default: 128, the whole job; 8 for --impl reference)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="c2", choices=sorted(WORKLOADS), help="c2 = BASELINE configs[1], the bench line")
@@ -581,16 +609,23 @@ def main():
     ap.add_argument("--with-c4", action="store_true", help="add the BASELINE configs[3] sub-record on one GPU too (always on for N > 1)")
     ap.add_argument("--no-c4", action="store_true")
     ap.add_argument("--c4-steps", type=int, default=6)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the accumulators of the timed path after its last step to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours (the reference arm only counts paths)")
     WORKLOAD.clear()
     WORKLOAD.update(WORKLOADS[args.workload])
     if args.passes_per_step <= 0:
         args.passes_per_step = WORKLOAD["passes_per_step"]
     if args.impl == "reference":
-        if args.steps == 128:
+        if args.steps is None:
             args.steps = 8  # each step is a bounded sample: keep the default run within minutes
         run_reference_arm(args)
     else:
+        if args.steps is None:
+            args.steps = 128
         if args.warmup < 3:
             args.warmup = 3  # timing rule: at least 3 warm-up steps
         run_ours(args)

@@ -38,6 +38,8 @@ static int fail(int code, const std::string& msg) {
     g_last_error = msg;
     return code;
 }
+// the same for the entry points defined in host/sample_scenes.cpp
+int ipt_host_fail(int code, const char* msg) { return fail(code, msg); }
 #define CUDA_TRY(expr)                                                                                           \
     do {                                                                                                         \
         cudaError_t e__ = (expr);                                                                                \

@@ -285,6 +285,8 @@ inline uint64_t splitmix64(uint64_t x) {
 
 } // namespace
 
+int ipt_host_fail(int code, const char* msg); // ipt_capi.cu: sets the calling thread's ipt_last_error()
+
 extern "C" {
 
 // Integer-defined mesh: every float is built from a 24-bit integer so that host, oracle and device inputs
@@ -335,7 +337,7 @@ int ipt_camera_orbit(ipt_camera* camera, int key) {
 }
 
 int ipt_sample_scene(const char* name, ipt_scene_desc** out) {
-    if (!name || !out) return IPT_ERR_INVALID;
+    if (!name || !out) return ipt_host_fail(IPT_ERR_INVALID, "ipt_sample_scene: name and out must not be null");
     std::string n(name);
     SceneHolder* s = new SceneHolder();
     std::memset(&s->desc, 0, sizeof(s->desc));
@@ -349,15 +351,15 @@ int ipt_sample_scene(const char* name, ipt_scene_desc** out) {
     else if (n == "mixedlights") scene_mixedlights(*s);
     else if (n.rfind("lightgrid:", 0) == 0) {
         int r = 0, c = 0;
-        if (std::sscanf(n.c_str() + 10, "%dx%d", &r, &c) != 2 || r <= 0 || c <= 0) { delete s; return IPT_ERR_INVALID; }
+        if (std::sscanf(n.c_str() + 10, "%dx%d", &r, &c) != 2 || r <= 0 || c <= 0) { delete s; return ipt_host_fail(IPT_ERR_INVALID, ("ipt_sample_scene: expected lightgrid:<rows>x<cols>, got " + n).c_str()); }
         scene_lightgrid(*s, r, c);
     } else if (n.rfind("mesh:", 0) == 0) {
         long long cnt = std::atoll(n.c_str() + 5);
-        if (cnt <= 0) { delete s; return IPT_ERR_INVALID; }
+        if (cnt <= 0) { delete s; return ipt_host_fail(IPT_ERR_INVALID, ("ipt_sample_scene: expected mesh:<triangles>, got " + n).c_str()); }
         scene_mesh(*s, (uint64_t)cnt);
     } else {
         delete s;
-        return IPT_ERR_INVALID;
+        return ipt_host_fail(IPT_ERR_INVALID, ("ipt_sample_scene: unknown scene " + n).c_str());
     }
     s->finish();
     *out = &s->desc;

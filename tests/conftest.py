@@ -31,13 +31,30 @@ def oracle():
 
 @pytest.fixture(scope="session")
 def ref():
-    """The compiled reference (oracle/_ref). Skips where neither the prebuilt .so nor /root/reference exists."""
+    """The compiled reference (oracle/_ref). Skips where neither the prebuilt .so nor the IPT_REFERENCE sources exist."""
     import oracle_lib
 
     r = oracle_lib.load_ref()
     if r is None:
-        pytest.skip("oracle/_ref/libipt_ref.so not available (no /root/reference to build it from)")
+        pytest.skip("oracle/_ref/libipt_ref.so not available (no IPT_REFERENCE sources to build it from)")
     return r
+
+
+@pytest.fixture(scope="session")
+def ref_or_none():
+    """The compiled reference where it is built, else None (tests then compare with its stored outputs)."""
+    import oracle_lib
+
+    return oracle_lib.load_ref()
+
+
+@pytest.fixture(scope="session")
+def pins():
+    """tests/golden/pin_live.npz: the reference's outputs the live pins compare with."""
+    import numpy as np
+    from helpers import PINS
+
+    return np.load(PINS)
 
 
 @pytest.fixture(scope="session")

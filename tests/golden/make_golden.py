@@ -14,6 +14,13 @@ Fixtures:
                      camera orbit on two input images (`python tests/golden/make_golden.py output`).
   image_<scene>.npz  sum / sumsq / count of the reference estimator (ray_power_recursive, n_rays=16, depth_max=4)
                      over P passes at WxH with libc drand48, merged over forked workers seeded 1000+rank.
+  pin_live.npz       what the bit-exact pins of tests/test_oracle_pin_live.py and tests/test_output_host.py compare the
+                     oracle with (`python tests/golden/make_golden.py pins`): whole drand48 passes (sha256 of pixels and
+                     counters, ray count, 4096 sampled pixels), mixture / DDF / light-DDF sample sequences, and the
+                     output stage on random ragged images. Recorded from the compiled reference. Where its sources are
+                     not at hand, `pins --from-oracle` records the oracle instead, which those pins held bit-identical
+                     to the reference; the file says which in `source`, and wherever the reference is built the tests
+                     check every stored array against it live.
 """
 from __future__ import annotations
 
@@ -161,6 +168,26 @@ def make_output_kat():
     np.savez_compressed(HERE / "output_kat.npz", **out)
 
 
+def make_pins():
+    import oracle_lib
+    import test_oracle_pin_live as P
+    import test_output_host as O
+
+    ref = oracle_lib.load_ref()
+    if ref is None and "--from-oracle" not in sys.argv:
+        raise SystemExit("the compiled reference (oracle/_ref/libipt_ref.so) is not built; `pins --from-oracle` records the oracle")
+    side, chk = ("ref", ref) if ref is not None else ("oracle", oracle_lib.load_oracle())
+    records = {P.pass_key(*c): P.pass_record(side, chk, *c) for c in P.PASS_CASES}
+    records.update({f"mix_{s}": P.mix_record(side, chk, s) for s in P.MIX_SCENES})
+    records.update({f"ddf_{k}": P.ddf_record(side, chk, k) for k in P.DDF_KINDS})
+    records.update({f"light_{s}": P.light_record(side, chk, s) for s in P.LIGHT_SCENES})
+    records["output"] = O.output_record(chk)
+    out = {f"{key}__{k}": v for key, rec in records.items() for k, v in rec.items()}
+    out["source"] = np.array("reference" if ref is not None else "oracle")
+    np.savez_compressed(HERE / "pin_live.npz", **out)
+    print("pin_live.npz:", len(out), "arrays from the", out["source"])
+
+
 if __name__ == "__main__":
     what = sys.argv[1] if len(sys.argv) > 1 else "all"
     if what in ("all", "kats"):
@@ -170,3 +197,5 @@ if __name__ == "__main__":
         make_images()
     if what in ("all", "kats", "output"):
         make_output_kat()
+    if what in ("all", "pins"):
+        make_pins()

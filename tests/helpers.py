@@ -1,6 +1,8 @@
 """Shared input generators for the parity tests."""
 from __future__ import annotations
 
+from pathlib import Path
+
 import numpy as np
 
 SCENES_REFERENCE = ["box", "fractal", "smallpt", "square", "corner", "openspheres"]
@@ -87,3 +89,36 @@ def block_sums(a, block):
     """Sums of block x block cells (frames whose sides are multiples of `block`)."""
     H, W = a.shape
     return a.reshape(H // block, block, W // block, block).sum((1, 3))
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# stored copies of the compiled reference's outputs (tests/golden/pin_live.npz, made by make_golden.py `pins`)
+# ---------------------------------------------------------------------------------------------------------------------
+PINS = Path(__file__).resolve().parent / "golden" / "pin_live.npz"
+
+
+def digest(a):
+    """sha256 of an array's bytes: bit-exact equality of frames too large to store."""
+    import hashlib
+
+    return np.array(hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest())
+
+
+def assert_same_record(got: dict, want: dict, what=""):
+    """Bit-exact equality of two records (same keys, dtypes, shapes and bytes)."""
+    assert sorted(got) == sorted(want), (what, sorted(got), sorted(want))
+    for k in want:
+        a, b = np.asarray(got[k]), np.asarray(want[k])
+        assert a.dtype == b.dtype and a.shape == b.shape and a.tobytes() == b.tobytes(), (what, k)
+
+
+def reference_record(pins, ref, key: str, from_ref):
+    """What the compiled reference gives for `key`. Where the reference is built (`ref` not None) it is run live and the
+    stored copy must equal it; elsewhere the stored copy stands in for it."""
+    stored = {k[len(key) + 2:]: pins[k] for k in pins.files if k.startswith(key + "__")}
+    assert stored, f"{key} missing from {PINS.name}: rerun `python tests/golden/make_golden.py pins`"
+    if ref is None:
+        return stored
+    live = {k: np.asarray(v) for k, v in from_ref(ref).items()}
+    assert_same_record(stored, live, f"stored {key} vs the live reference")
+    return live

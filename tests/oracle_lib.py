@@ -1,8 +1,8 @@
 """ctypes access to the two CPU checkers — TEST INFRASTRUCTURE, importable from tests/, smoke() and bench.py only.
 
 * oracle/libipt_oracle.so — our plain-C restatement (oracle/ipt_oracle.c), built with `make -C oracle oracle`.
-* oracle/_ref/libipt_ref.so — the unmodified reference compiled from /root/reference (`make -C oracle ref`);
-  on the GPU box only the prebuilt file exists (it travels with the snapshot).
+* oracle/_ref/libipt_ref.so — the unmodified reference compiled from the dimalit/ipt checkout that IPT_REFERENCE names
+  (`make -C oracle ref REF=...`); where none is given, a prebuilt file is used if present.
 """
 from __future__ import annotations
 
@@ -16,7 +16,7 @@ import numpy as np
 ROOT = Path(__file__).resolve().parent.parent
 ORACLE_SO = ROOT / "oracle" / "libipt_oracle.so"
 REF_SO = ROOT / "oracle" / "_ref" / "libipt_ref.so"
-REF_SRC = Path(os.environ.get("IPT_REFERENCE", "/root/reference"))
+REF_SRC = Path(os.environ["IPT_REFERENCE"]) if os.environ.get("IPT_REFERENCE") else None  # not part of this repository
 
 f32p = C.POINTER(C.c_float)
 f64p = C.POINTER(C.c_double)
@@ -44,7 +44,7 @@ def build_oracle():
 
 def build_ref():
     """Compiles the reference where it lies; returns None if it is neither built nor buildable here."""
-    if REF_SRC.exists():
+    if REF_SRC is not None and REF_SRC.exists():
         if _stale(REF_SO, [ROOT / "oracle" / "ref_driver.cpp", ROOT / "oracle" / "ref_gui_driver.cpp"]):
             subprocess.run(["make", "-C", str(ROOT / "oracle"), "ref", f"REF={REF_SRC}"], check=True, capture_output=True)
     return REF_SO if REF_SO.exists() else None
@@ -56,7 +56,7 @@ DROPIN = ROOT / "oracle" / "_ref" / "ab_dropin"
 def build_dropin():
     """oracle/_ref/ab_dropin (ipt_b200's host classes compiled against the reference's headers + the reference's own
     estimator): built where the reference sources exist, else the prebuilt binary if it travelled with the snapshot."""
-    if REF_SRC.exists() and (ROOT / "ipt_b200" / "lib" / "libipt_b200.so").exists():
+    if REF_SRC is not None and REF_SRC.exists() and (ROOT / "ipt_b200" / "lib" / "libipt_b200.so").exists():
         deps = [ROOT / "oracle" / "ab_dropin.cpp", ROOT / "ipt_b200" / "host" / "device_plugins.cpp", ROOT / "ipt_b200" / "host" / "device_plugins.hpp", REF_SO]
         if _stale(DROPIN, deps):
             subprocess.run(["make", "-C", str(ROOT / "oracle"), "ref", "dropin", f"REF={REF_SRC}"], check=True, capture_output=True)

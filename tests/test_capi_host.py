@@ -76,10 +76,11 @@ def test_sample_scene_names_and_errors(lib):
         assert (sd.desc.n_prims, sd.desc.n_lights) == (prims, lights), name
     assert capi.SceneDescription("fractal").desc.n_prims == 7  # FractalSpheres prints 7 spheres (r >= 0.001)
     for bad in ["nope", "mesh:0", "lightgrid:0x3", "lightgrid:abc"]:
-        with pytest.raises(capi.IptError):
+        with pytest.raises(capi.IptError, match=bad):
             capi.SceneDescription(bad)
     out = C.POINTER(capi.SceneDesc)()
-    assert lib.ipt_sample_scene(None, C.byref(out)) != 0 and b"" != lib.ipt_last_error()
+    # the message is this call's own, not one left on the thread by an earlier failure
+    assert lib.ipt_sample_scene(None, C.byref(out)) != 0 and b"ipt_sample_scene" in lib.ipt_last_error()
 
 
 def test_generated_mesh_is_integer_defined(lib):

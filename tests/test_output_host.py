@@ -1,6 +1,7 @@
 """Output stage (src/gui.cpp) on the CPU side: the oracle restatement against the reference's golden vectors
-(tests/golden/output_kat.npz, made by make_golden.py from the compiled gui.cpp) and live against the compiled reference;
-the product's host-only pieces (camera orbit, PNG writer); and the no-GPU error behaviour of the device entry points."""
+(tests/golden/output_kat.npz, made by make_golden.py from the compiled gui.cpp) and against the compiled reference, live
+or through its stored outputs (tests/golden/pin_live.npz); the product's host-only pieces (camera orbit, PNG writer);
+and the no-GPU error behaviour of the device entry points."""
 import struct
 import zlib
 from pathlib import Path
@@ -8,7 +9,7 @@ from pathlib import Path
 import numpy as np
 import pytest
 
-from helpers import bits
+from helpers import assert_same_record, bits, reference_record
 from ipt_b200 import capi
 
 GOLD = Path(__file__).resolve().parent / "golden"
@@ -36,22 +37,32 @@ def test_oracle_camera_orbit_equals_reference_golden(kat, oracle):
         assert np.array_equal(bits(got), bits(cams[i + 1])), (i, k)
 
 
-def test_oracle_output_stage_live_against_reference(oracle, ref):
-    """Random images, ragged sizes: every function of the restatement is bit-identical to the compiled gui.cpp."""
+def output_record(chk):
+    """Random images, ragged sizes: normalize(), Gui::save bytes and glare() of src/gui.cpp, and a run of camera keys, on
+    either checker (the oracle or the compiled reference: same interface)."""
     rng = np.random.default_rng(17)
+    out = {}
     for (h, w) in [(1, 1), (3, 5), (40, 57), (64, 64)]:
         img = (rng.random((h, w)).astype(np.float32) ** 5 * np.float32(6.0)).astype(np.float32)
         img[rng.random((h, w)) < 0.3] = 0
         img.flat[0] = 2.5  # never black
-        assert np.array_equal(bits(oracle.image_normalize(img)), bits(ref.image_normalize(img)))
-        assert np.array_equal(oracle.image_save_bytes(img), ref.image_save_bytes(img))
+        out[f"normalize_{h}x{w}"] = bits(chk.image_normalize(img))
+        out[f"bytes_{h}x{w}"] = chk.image_save_bytes(img)
         for c in [1.01, 0.4, 100.0]:
-            assert np.array_equal(bits(oracle.image_glare(img, c)), bits(ref.image_glare(img, c))), (h, w, c)
+            out[f"glare_{h}x{w}_{c}"] = bits(chk.image_glare(img, c))
     pos, d = np.array([1.5, -2.0, 0.7], np.float32), np.array([-0.3, 0.9, -0.2], np.float32)
-    for k in [0, 1, 2, 3, 1, 1, 3, 0]:
-        a, b = oracle.camera_orbit(pos, d, k), ref.camera_orbit(pos, d, k)
-        assert np.array_equal(bits(a), bits(b))
-        pos, d = a[0], a[1]
+    for i, k in enumerate([0, 1, 2, 3, 1, 1, 3, 0]):
+        cam = chk.camera_orbit(pos, d, k)
+        out[f"orbit_{i}"] = bits(cam)
+        pos, d = cam[0], cam[1]
+    return out
+
+
+def test_oracle_output_stage_live_against_reference(oracle, ref_or_none, pins):
+    """Every function of the restatement is bit-identical to the compiled gui.cpp: live where the reference is built,
+    else against its stored outputs (tests/golden/pin_live.npz)."""
+    want = reference_record(pins, ref_or_none, "output", output_record)
+    assert_same_record(output_record(oracle), want)
 
 
 def test_product_camera_orbit_bit_exact(kat, lib):
