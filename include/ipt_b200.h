@@ -196,6 +196,18 @@ int ipt_scene_create(const ipt_scene_desc* desc, int device, ipt_scene** out);
 int ipt_scene_destroy(ipt_scene* scene);
 /* SimpleCamera can be orbited by the caller (gui.cpp:107-137): replace the camera without a rebuild. */
 int ipt_scene_set_camera(ipt_scene* scene, const ipt_camera* camera);
+/* Which kernel instantiations ipt_scene_create chose for the scene (read-only; renders do not depend on it):
+ *   out[0] spec of the fused shade kernels: 0 FEW_LIGHTS (no light LBVH; the lights are scanned from global memory),
+ *          1 LIGHT_BVH (more than 8 lights, all of them area lights), 2 RUNTIME (SmallPt scenes: decided per call),
+ *          3 ONE_LIGHT (one light, not an area light), 4 ONE_AREA_LIGHT (one area light), 5 BOX_SCENE (... and the
+ *          geometry is grouped box planes + inline spheres), 6 LAMBERT_BOX (... and every material is the cosine DDF)
+ *   out[1] SmallPt spheres present, out[2] triangle mesh present: together they select k_extend<smallpt, mesh>
+ *   out[3] mesh scene traced by the box-scene mesh kernel (k_extend_mesh<., BOX_SCENE>) instead of the generic one
+ *   out[4] shadow rays skip the box walls (every sphere inside the box, every area-light corner 1e-3 from the walls)
+ *   out[5] the lights are held in kernel parameters (a single light)
+ *   out[6] number of lights in the light LBVH (0: none) */
+#define IPT_DISPATCH_WORDS 7
+int ipt_scene_dispatch(ipt_scene* scene, uint32_t out[IPT_DISPATCH_WORDS]);
 
 /* The reference's five scenes + this repo's benchmark scenes as descriptions:
  * "box" (make_scene_box, the default), "fractal", "smallpt", "square", "corner", "openspheres", "cornell" (C2),

@@ -17,6 +17,10 @@ FLAG_TIME_KERNELS, FLAG_KEEP_ZERO_WEIGHT, FLAG_DEBUG_PRINT, FLAG_RESOLVE_LAST_LE
 STATUS = {0: "IPT_OK", 1: "IPT_ERR_INVALID", 2: "IPT_ERR_CUDA", 3: "IPT_ERR_NO_DEVICE", 4: "IPT_ERR_UNSUPPORTED", 5: "IPT_ERR_OVERFLOW"}
 IPT_ERR_INVALID = 1
 IPT_ERR_NO_DEVICE = 3
+# ipt_scene_dispatch: out[0] names the shade spec, the other words are flags / counts
+SPEC_FEW_LIGHTS, SPEC_LIGHT_BVH, SPEC_RUNTIME, SPEC_ONE_LIGHT, SPEC_ONE_AREA_LIGHT, SPEC_BOX_SCENE, SPEC_LAMBERT_BOX = range(7)
+DISPATCH_FIELDS = ("spec", "smallpt", "mesh", "mesh_box_scene", "lights_inside_box", "light_inline", "n_light_bvh")
+DISPATCH_WORDS = len(DISPATCH_FIELDS)
 
 import os
 
@@ -95,6 +99,7 @@ SIGNATURES = {
     "ipt_scene_create": (C.c_int, [C.POINTER(SceneDesc), C.c_int, C.POINTER(_vp)]),
     "ipt_scene_destroy": (C.c_int, [_vp]),
     "ipt_scene_set_camera": (C.c_int, [_vp, C.POINTER(Camera)]),
+    "ipt_scene_dispatch": (C.c_int, [_vp, u32p]),
     "ipt_sample_scene": (C.c_int, [C.c_char_p, C.POINTER(C.POINTER(SceneDesc))]),
     "ipt_scene_desc_free": (C.c_int, [C.POINTER(SceneDesc)]),
     "ipt_light_derived": (C.c_int, [C.POINTER(Light), f32p, f32p, f32p]),
@@ -277,6 +282,12 @@ class Scene:
             self.close()
         except Exception:
             pass
+
+    def dispatch(self) -> dict:
+        """ipt_scene_dispatch: the kernel instantiations ipt_scene_create chose (see include/ipt_b200.h)."""
+        out = np.zeros(DISPATCH_WORDS, np.uint32)
+        check(load().ipt_scene_dispatch(self.handle, _ptr(out, u32p)))
+        return dict(zip(DISPATCH_FIELDS, (int(v) for v in out)))
 
     def trace_batch(self, origins, directions):
         o, d = _f32(origins).reshape(-1, 3), _f32(directions).reshape(-1, 3)

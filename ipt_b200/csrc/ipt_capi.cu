@@ -716,6 +716,27 @@ int ipt_scene_set_camera(ipt_scene* s, const ipt_camera* camera) {
     return IPT_OK;
 }
 
+int ipt_scene_dispatch(ipt_scene* s, uint32_t out[IPT_DISPATCH_WORDS]) {
+    if (!s || !out) return fail(IPT_ERR_INVALID, "null argument");
+    std::lock_guard<std::recursive_mutex> lock__(s->mu);
+    // the same chain of predicates as the fused k_shade launches of ipt_render
+    const SceneSpec spec = s->smallpt ? SPEC_RUNTIME
+                           : s->dev.n_light_bvh ? SPEC_LIGHT_BVH
+                           : (s->inline_area_light && s->geom_fast && s->all_lambert) ? SPEC_LAMBERT_BOX
+                           : (s->inline_area_light && s->geom_fast) ? SPEC_BOX_SCENE
+                           : s->inline_area_light ? SPEC_ONE_AREA_LIGHT
+                           : s->dev.light_inline ? SPEC_ONE_LIGHT
+                                                 : SPEC_FEW_LIGHTS;
+    out[0] = (uint32_t)spec;
+    out[1] = s->smallpt;
+    out[2] = s->mesh;
+    out[3] = s->mesh_box_scene;
+    out[4] = s->dev.lights_inside_box;
+    out[5] = s->dev.light_inline;
+    out[6] = s->dev.n_light_bvh;
+    return IPT_OK;
+}
+
 // ---- parity entries ----------------------------------------------------------------------------------
 int ipt_trace_batch(ipt_scene* s, const float* origins, const float* directions, size_t n, uint32_t* prim_id, float* t,
                     uint32_t* light_id, float* light_pos, uint32_t* outcome) {

@@ -122,3 +122,45 @@ def reference_record(pins, ref, key: str, from_ref):
     live = {k: np.asarray(v) for k, v in from_ref(ref).items()}
     assert_same_record(stored, live, f"stored {key} vs the live reference")
     return live
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# scenes built in Python on top of a sample scene
+# ---------------------------------------------------------------------------------------------------------------------
+def custom_scene(base="box", prims=None, lights=None, materials=None, triangles=None, triangle_material=None):
+    """A library-owned description of `base` with some of its arrays replaced by Python-built ones (kept alive by the
+    description)."""
+    from ipt_b200 import capi
+
+    sd = capi.SceneDescription(base)
+    keep = []
+    if prims is not None:
+        arr = (capi.Prim * len(prims))(*prims)
+        sd.desc.prims, sd.desc.n_prims = arr, len(prims)
+        keep.append(arr)
+    if lights is not None:
+        arr = (capi.Light * len(lights))(*lights)
+        sd.desc.lights, sd.desc.n_lights = arr, len(lights)
+        keep.append(arr)
+    if materials is not None:
+        arr = (capi.Material * len(materials))(*materials)
+        sd.desc.materials, sd.desc.n_materials = arr, len(materials)
+        keep.append(arr)
+    if triangles is not None:
+        tris = np.ascontiguousarray(triangles, np.float32).reshape(-1, 9)
+        sd.desc.triangles, sd.desc.n_triangles = tris.ctypes.data_as(capi.f32p), tris.shape[0]
+        keep.append(tris)
+    if triangle_material is not None:
+        sd.desc.triangle_material = triangle_material
+    sd._keep = keep
+    return sd
+
+
+def make_light(kind, position, x_axis=(0, 0, 0), y_axis=(0, 0, 0), radius=0.0, power=1.0):
+    from ipt_b200 import capi
+
+    l = capi.Light()
+    l.kind = kind
+    l.position[:] = [float(v) for v in position]; l.x_axis[:] = [float(v) for v in x_axis]; l.y_axis[:] = [float(v) for v in y_axis]
+    l.radius = radius; l.power = power
+    return l

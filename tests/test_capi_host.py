@@ -36,7 +36,7 @@ def test_enum_values_and_struct_sizes_against_a_c_compiler(lib, tmp_path):
 
     names = ["IPT_FLAG_TIME_KERNELS", "IPT_FLAG_KEEP_ZERO_WEIGHT", "IPT_FLAG_DEBUG_PRINT", "IPT_FLAG_RESOLVE_LAST_LEVEL",
              "IPT_FLAG_NO_FUSED_LAST_LEVEL", "IPT_FLAG_NO_FUSED_TRACE", "IPT_PLANE_GRID", "IPT_PLANE_GUI", "IPT_PLANE_LINEAR",
-             "IPT_KEY_LEFT", "IPT_KEY_RIGHT", "IPT_KEY_DOWN", "IPT_KEY_UP", "IPT_ERR_INVALID", "IPT_ERR_NO_DEVICE", "IPT_MAX_DEPTH"]
+             "IPT_KEY_LEFT", "IPT_KEY_RIGHT", "IPT_KEY_DOWN", "IPT_KEY_UP", "IPT_ERR_INVALID", "IPT_ERR_NO_DEVICE", "IPT_MAX_DEPTH", "IPT_DISPATCH_WORDS"]
     structs = ["ipt_material", "ipt_prim", "ipt_light", "ipt_camera", "ipt_scene_desc", "ipt_render_params", "ipt_render_stats", "ipt_bvh_node"]
     src = tmp_path / "probe.c"
     src.write_text('#include <stdio.h>\n#include "ipt_b200.h"\nint main(void) {\n'
@@ -52,6 +52,7 @@ def test_enum_values_and_struct_sizes_against_a_c_compiler(lib, tmp_path):
             "IPT_PLANE_GRID": capi.PLANE_GRID, "IPT_PLANE_GUI": capi.PLANE_GUI, "IPT_PLANE_LINEAR": capi.PLANE_LINEAR,
             "IPT_KEY_LEFT": 0, "IPT_KEY_RIGHT": 1, "IPT_KEY_DOWN": 2, "IPT_KEY_UP": 3,
             "IPT_ERR_INVALID": capi.IPT_ERR_INVALID, "IPT_ERR_NO_DEVICE": capi.IPT_ERR_NO_DEVICE, "IPT_MAX_DEPTH": capi.IPT_MAX_DEPTH,
+            "IPT_DISPATCH_WORDS": capi.DISPATCH_WORDS,
             "sizeof_ipt_material": C.sizeof(capi.Material), "sizeof_ipt_prim": C.sizeof(capi.Prim), "sizeof_ipt_light": C.sizeof(capi.Light),
             "sizeof_ipt_camera": C.sizeof(capi.Camera), "sizeof_ipt_scene_desc": C.sizeof(capi.SceneDesc),
             "sizeof_ipt_render_params": C.sizeof(capi.RenderParams), "sizeof_ipt_render_stats": C.sizeof(capi.RenderStats),

@@ -7,7 +7,7 @@ import numpy as np
 import pytest
 
 import oracle_lib
-from helpers import SCENES_ANALYTIC, bits, ray_batch
+from helpers import SCENES_ANALYTIC, bits, custom_scene, ray_batch
 from ipt_b200 import capi
 
 pytestmark = pytest.mark.gpu
@@ -106,13 +106,29 @@ def test_two_level_render_matches_oracle_per_pixel(name, res, scenes, oracle):
                                        flags=capi.FLAG_KEEP_ZERO_WEIGHT)
     assert np.array_equal(cnt.astype(np.uint64), o["counters"])
     assert st.paths == res * res * 2
-    ref = o["sum"]
-    scale = max(ref.max(), 1e-12)
-    err = np.abs(s - ref) / scale
-    assert (err > 1e-5).mean() < 4e-3, f"{(err > 1e-5).sum()} pixels differ"
-    assert abs(s.sum() - ref.sum()) <= 1e-4 * max(ref.sum(), 1e-9)
+    # sum and sumsq (what checkpoints and bench.py --dump-outputs carry) against the oracle's double accumulators; a square
+    # doubles relative differences, hence twice the bound on the sumsq total
+    for got, ref, total in ((s, o["sum"], 1e-4), (q, o["sumsq"], 2e-4)):
+        scale = max(ref.max(), 1e-12)
+        err = np.abs(got - ref) / scale
+        assert (err > 1e-5).mean() < 4e-3, f"{(err > 1e-5).sum()} pixels differ"
+        assert abs(got.sum() - ref.sum()) <= total * max(ref.sum(), 1e-9)
     assert abs(int(st.rays) - int(o["rays"])) <= 2e-4 * o["rays"] + 2
     assert st.rays_at_depth[0] == o["rays_at_depth"][0] == res * res * 2
+
+
+def test_gui_plane_two_level_render_matches_oracle_per_pixel(scenes, oracle):
+    """IPT_PLANE_GUI (Gui::addRay's cell mapping, gui.cpp:168-172) through the whole render: counters, sum and sumsq per
+    cell against the oracle, which maps its samples the same way."""
+    sd, sc = scenes("cornell")
+    p, s, q, cnt, st, o = _render_pair(sd, sc, oracle, width=64, height=48, pass_count=2, depth_max=2, schedule=[16, 8],
+                                       plane_mode=capi.PLANE_GUI, flags=capi.FLAG_KEEP_ZERO_WEIGHT)
+    assert np.array_equal(cnt.astype(np.uint64), o["counters"])
+    for got, ref, total in ((s, o["sum"], 1e-4), (q, o["sumsq"], 2e-4)):
+        scale = max(ref.max(), 1e-12)
+        err = np.abs(got - ref) / scale
+        assert (err > 1e-5).mean() < 4e-3, f"{(err > 1e-5).sum()} pixels differ"
+        assert abs(got.sum() - ref.sum()) <= total * max(ref.sum(), 1e-9)
 
 
 @pytest.mark.parametrize("name,res", [("box", 96), ("cornell", 96), ("corner", 64), ("smallpt", 48), ("lightgrid:3x3", 48)])
@@ -345,32 +361,6 @@ def test_edge_cases_and_argument_validation(scenes, oracle):
         capi.Scene(sd2)
 
 
-def _custom_scene(prims=None, lights=None, base="box"):
-    """A library-owned description with its primitive / light arrays replaced by Python-built ones (kept alive)."""
-    sd = capi.SceneDescription(base)
-    keep = []
-    if prims is not None:
-        arr = (capi.Prim * len(prims))(*prims)
-        sd.desc.prims = arr
-        sd.desc.n_prims = len(prims)
-        keep.append(arr)
-    if lights is not None:
-        arr = (capi.Light * len(lights))(*lights)
-        sd.desc.lights = arr
-        sd.desc.n_lights = len(lights)
-        keep.append(arr)
-    sd._keep = keep
-    return sd
-
-
-def _light(kind, position, x_axis=(0, 0, 0), y_axis=(0, 0, 0), radius=0.0, power=1.0):
-    l = capi.Light()
-    l.kind = kind
-    l.position[:] = position; l.x_axis[:] = x_axis; l.y_axis[:] = y_axis
-    l.radius = radius; l.power = power
-    return l
-
-
 def test_every_light_kind_in_one_collection(lib, oracle):
     """CollectionLighting with all five Light classes at once (lighting.h:16-73, CollectionLighting.cpp:36-55): square,
     triangle, sphere, inverted sphere ("outer light") and point light. Mixed kinds take the linear multi-light path."""
@@ -431,7 +421,7 @@ def test_many_spheres_take_the_generic_primitive_scan(lib, oracle):
         pr.radius = float(rng.uniform(0.05, 0.2)); pr.curvature = 1.0 / pr.radius
         prims.append(pr)
     prims.append(prims[7])  # an exact duplicate: the first one must keep winning
-    sd = _custom_scene(prims=prims)
+    sd = custom_scene(prims=prims)
     sc = capi.Scene(sd)
     o, d, _ = ray_batch("box", lambda xy: oracle.camera_rays(sd.ptr, xy), n_cam_side=64, n_random=20000)
     g = sc.trace_batch(o, d); c = oracle.trace_batch(sd.ptr, o, d)
