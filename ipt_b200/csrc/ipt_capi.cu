@@ -18,16 +18,12 @@
 #include <cstring>
 #include <mutex>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 using namespace iptd;
 
 #define IPT_LIGHT_BVH_MIN 8 // light sets larger than this get an LBVH
-#ifndef IPT_RENDER_LANES
-#define IPT_RENDER_LANES 1 // 2: mesh scenes keep two batches in flight on two streams (ipt_render). Measured (profiles/tuning_r02.md):
-                           // C3 397 -> 411, C4 339 -> 347 Mpaths/s with two full 2^25-path batches, nothing when the job has to be
-                           // split in two for it, and per-kernel CUDA-event times lose their meaning under the overlap: off
-#endif
 #define IPT_CNT_WORDS (3 * IPT_MAX_DEPTH + 2) // ray counts, hit counts, persistent-kernel fetch cursors
 
 // ---------------------------------------------------------------------------------------------------
@@ -96,6 +92,15 @@ struct OutputScratch {
     GrowBuf mean, glare, shown, bytes, rows, bright, small;
 };
 
+// One kernel of ipt_render's depth loop (k_extend, k_extend_mesh or k_shade), the grid its own occupancy allows and its
+// dynamic shared memory
+struct RenderKernel {
+    using Fn = void (*)(DevScene, RenderCtx, uint32_t);
+    Fn kernel = nullptr;
+    int grid = 0;
+    size_t smem = 0;
+};
+
 struct ipt_scene {
     // The reference calls render_sample from four threads on one Scene (main.cpp:258-277). One scene owns one stream and
     // one workspace, so every entry point that touches them takes this lock: concurrent callers are serialised.
@@ -113,14 +118,11 @@ struct ipt_scene {
     LbvhDevice bvh{};
     LbvhDevice light_bvh{};
     bool smallpt = false, mesh = false;
-    bool inline_area_light = false; // the scene's lights are the inline ones and all of them are area lights
-    bool geom_fast = false;         // grouped box planes + inline spheres only (analytic_closest's first branch)
-    bool all_lambert = false;       // every material is the cosine DDF
-    bool mesh_box_scene = false;    // mesh scene whose lights / analytic primitives allow k_extend_mesh<.., SPEC_BOX_SCENE>
+    SceneSpec shade_spec = SPEC_RUNTIME; // k_shade<FUSE_NEXT / FUSE_LAST, ., shade_spec>
+    SceneSpec mesh_spec = SPEC_RUNTIME;  // k_extend_mesh<., mesh_spec> (mesh scenes without SmallPt)
+    // the kernels of ipt_render's depth loop, chosen once by ipt_scene_create; extend[last depth][exact arithmetic]
+    RenderKernel extend[2][2], shade, shade_next, shade_last;
     Workspace ws;
-    Workspace ws2;                  // second lane of ipt_render (mesh scenes: two batches in flight, see ipt_render)
-    cudaStream_t stream2 = nullptr;
-    cudaEvent_t ev_join = nullptr;
     uint32_t* d_cnt = nullptr;
     unsigned long long* d_stats = nullptr;
     std::vector<cudaEvent_t> events;
@@ -128,8 +130,7 @@ struct ipt_scene {
     ipt_plane* host_plane = nullptr; // for ipt_render_host
     float* pinned = nullptr;         // staging for ipt_render_host
     size_t pinned_bytes = 0;
-    int grid_mesh = 0, grid_mesh_last = 0;
-    int grid_generate = 0, grid_extend = 0, grid_extend_last = 0, grid_shade = 0, grid_shade_fused = 0, grid_shade_next = 0, grid_accumulate = 0;
+    int grid_generate = 0, grid_accumulate = 0;
     OutputScratch out;
 };
 
@@ -409,16 +410,30 @@ static int occupancy_grid(K kernel, int sm_count, size_t smem) {
     return sm_count * per_sm;
 }
 
-#define DISPATCH_SM(scene, CALL)                         \
-    do {                                                 \
-        if ((scene)->smallpt && (scene)->mesh) { CALL(true, true); }        \
-        else if ((scene)->smallpt) { CALL(true, false); }                   \
-        else if ((scene)->mesh) { CALL(false, true); }                      \
-        else { CALL(false, false); }                                        \
-    } while (0)
+// f(smallpt, mesh) with the scene's two flags as std::bool_constant, for the kernels compiled per <SMALLPT, MESH>
+template <class F>
+static void with_scene_kind(const ipt_scene* s, F&& f) {
+    if (s->smallpt && s->mesh) f(std::true_type{}, std::true_type{});
+    else if (s->smallpt) f(std::true_type{}, std::false_type{});
+    else if (s->mesh) f(std::false_type{}, std::true_type{});
+    else f(std::false_type{}, std::false_type{});
+}
+
+// the fused k_shade of a scene spec; SPEC_RUNTIME is the SmallPt kernel, which keeps the runtime light switch
+template <int FUSE>
+static RenderKernel::Fn fused_shade(SceneSpec spec) {
+    switch (spec) {
+        case SPEC_LIGHT_BVH: return k_shade<FUSE, false, SPEC_LIGHT_BVH>;
+        case SPEC_LAMBERT_BOX: return k_shade<FUSE, false, SPEC_LAMBERT_BOX>;
+        case SPEC_BOX_SCENE: return k_shade<FUSE, false, SPEC_BOX_SCENE>;
+        case SPEC_ONE_AREA_LIGHT: return k_shade<FUSE, false, SPEC_ONE_AREA_LIGHT>;
+        case SPEC_ONE_LIGHT: return k_shade<FUSE, false, SPEC_ONE_LIGHT>;
+        case SPEC_FEW_LIGHTS: return k_shade<FUSE, false, SPEC_FEW_LIGHTS>;
+        default: return k_shade<FUSE, true>;
+    }
+}
 
 static size_t stack_smem(const ipt_scene* s) { return s->mesh ? (size_t)IPT_STACK_SHORT * IPT_BLOCK * sizeof(uint32_t) : 0; }
-static size_t mesh_smem(const ipt_scene* s) { return s->mesh ? (size_t)IPT_MESH_SMEM_BYTES : 0; } // k_extend_mesh: stacks + the per-warp ray pools
 
 template <class T>
 struct DevBuf {
@@ -512,9 +527,9 @@ int ipt_scene_create(const ipt_scene_desc* desc, int device, ipt_scene** out) {
     dv.sdf_weight = sdf_weight;
     dv.prim_inline = desc->n_prims <= IPT_INLINE_PRIMS;
     dv.light_inline = desc->n_lights <= IPT_INLINE_LIGHTS;
-    s->inline_area_light = dv.light_inline && desc->n_lights > 0;
+    bool inline_area_light = dv.light_inline && desc->n_lights > 0; // the lights are the inline ones, all of them area lights
     for (uint32_t i = 0; i < desc->n_lights && i < IPT_INLINE_LIGHTS; ++i)
-        if (desc->lights[i].kind > IPT_LIGHT_AREA_TRIANGLE) s->inline_area_light = false;
+        if (desc->lights[i].kind > IPT_LIGHT_AREA_TRIANGLE) inline_area_light = false;
     auto upload = [&](auto*& dptr, const auto& vec) -> cudaError_t {
         size_t bytes = std::max<size_t>(vec.size(), 1) * sizeof(vec[0]);
         cudaError_t e = cudaMalloc((void**)&dptr, bytes);
@@ -579,12 +594,13 @@ int ipt_scene_create(const ipt_scene_desc* desc, int device, ipt_scene** out) {
     set_camera(dv, desc->camera);
     s->smallpt = smallpt;
     s->mesh = desc->n_triangles > 0;
-    s->geom_fast = !smallpt && !s->mesh && dv.planes_grouped && dv.others_inline;
+    // grouped box planes + inline spheres only (analytic_closest's first branch)
+    const bool geom_fast = !smallpt && !s->mesh && dv.planes_grouped && dv.others_inline;
     // Shadow rays of box scenes skip the wall planes (DevScene::lights_inside_box): every non-plane primitive is a sphere
     // inside the closed box [-1,1]^3 and every light is an area light whose corners keep a margin of 1e-3 to every wall, so
     // origin (a point of a wall or of a sphere) and target lie in the convex box and no wall can come between them.
     dv.lights_inside_box = 0;
-    if (s->geom_fast && s->inline_area_light && dv.n_planes > 0) {
+    if (geom_fast && inline_area_light && dv.n_planes > 0) {
         bool inside = true;
         for (uint32_t k = 0; k < dv.n_others; ++k) {
             const DevSphere& sp = dv.others[k];
@@ -601,8 +617,8 @@ int ipt_scene_create(const ipt_scene_desc* desc, int device, ipt_scene** out) {
         }
         dv.lights_inside_box = inside ? 1u : 0u;
     }
-    s->all_lambert = true;
-    for (const DevMaterial& m : mats) if (m.ddf != IPT_DDF_COSINE) s->all_lambert = false;
+    bool all_lambert = true; // every material is the cosine DDF
+    for (const DevMaterial& m : mats) if (m.ddf != IPT_DDF_COSINE) all_lambert = false;
     if (s->mesh) {
         std::string err;
         if (lbvh_build(desc->triangles, (uint32_t)desc->n_triangles, s->stream, s->bvh, err) != 0)
@@ -640,41 +656,40 @@ int ipt_scene_create(const ipt_scene_desc* desc, int device, ipt_scene** out) {
             dv.n_light_bvh = desc->n_lights;
         }
     }
-    CUDA_TRY(cudaMalloc((void**)&s->d_cnt, sizeof(uint32_t) * IPT_CNT_WORDS * 2)); // one set of queue counters per lane of ipt_render
-    CUDA_TRY(cudaStreamCreateWithFlags(&s->stream2, cudaStreamNonBlocking));
-    CUDA_TRY(cudaEventCreateWithFlags(&s->ev_join, cudaEventDisableTiming));
+    CUDA_TRY(cudaMalloc((void**)&s->d_cnt, sizeof(uint32_t) * IPT_CNT_WORDS));
     CUDA_TRY(cudaMalloc((void**)&s->d_stats, sizeof(unsigned long long) * ST_COUNT));
 
-    size_t sm = stack_smem(s);
+    // the kernels compiled for this kind of scene (SceneSpec in ipt_kernels.cuh)
+    s->shade_spec = smallpt ? SPEC_RUNTIME
+                    : dv.n_light_bvh ? SPEC_LIGHT_BVH
+                    : (inline_area_light && geom_fast && all_lambert) ? SPEC_LAMBERT_BOX
+                    : (inline_area_light && geom_fast) ? SPEC_BOX_SCENE
+                    : inline_area_light ? SPEC_ONE_AREA_LIGHT
+                    : dv.light_inline ? SPEC_ONE_LIGHT
+                                      : SPEC_FEW_LIGHTS;
+    const bool persistent_mesh = s->mesh && !smallpt;
+    s->mesh_spec = persistent_mesh && inline_area_light && dv.planes_grouped && dv.others_inline ? SPEC_BOX_SCENE : SPEC_RUNTIME;
+    auto entry = [&](RenderKernel::Fn k, size_t smem) { return RenderKernel{k, occupancy_grid(k, s->sm_count, smem), smem}; };
     s->grid_generate = occupancy_grid(k_generate, s->sm_count, 0);
-    s->grid_shade = occupancy_grid(k_shade<FUSE_NONE, false>, s->sm_count, 0);
-    // (SmallPt scenes keep the runtime light switch; the others get the kernel compiled for their kind of light set)
-    s->grid_shade_fused = s->smallpt ? occupancy_grid(k_shade<FUSE_LAST, true>, s->sm_count, 0)
-                          : dv.n_light_bvh ? occupancy_grid(k_shade<FUSE_LAST, false, SPEC_LIGHT_BVH>, s->sm_count, 0)
-                          : (s->inline_area_light && s->geom_fast && s->all_lambert) ? occupancy_grid(k_shade<FUSE_LAST, false, SPEC_LAMBERT_BOX>, s->sm_count, 0)
-                          : (s->inline_area_light && s->geom_fast) ? occupancy_grid(k_shade<FUSE_LAST, false, SPEC_BOX_SCENE>, s->sm_count, 0)
-                          : s->inline_area_light ? occupancy_grid(k_shade<FUSE_LAST, false, SPEC_ONE_AREA_LIGHT>, s->sm_count, 0)
-                          : dv.light_inline ? occupancy_grid(k_shade<FUSE_LAST, false, SPEC_ONE_LIGHT>, s->sm_count, 0)
-                                            : occupancy_grid(k_shade<FUSE_LAST, false, SPEC_FEW_LIGHTS>, s->sm_count, 0);
-    s->grid_shade_next = s->smallpt ? occupancy_grid(k_shade<FUSE_NEXT, true>, s->sm_count, 0)
-                         : dv.n_light_bvh ? occupancy_grid(k_shade<FUSE_NEXT, false, SPEC_LIGHT_BVH>, s->sm_count, 0)
-                         : (s->inline_area_light && s->geom_fast && s->all_lambert) ? occupancy_grid(k_shade<FUSE_NEXT, false, SPEC_LAMBERT_BOX>, s->sm_count, 0)
-                          : (s->inline_area_light && s->geom_fast) ? occupancy_grid(k_shade<FUSE_NEXT, false, SPEC_BOX_SCENE>, s->sm_count, 0)
-                          : s->inline_area_light ? occupancy_grid(k_shade<FUSE_NEXT, false, SPEC_ONE_AREA_LIGHT>, s->sm_count, 0)
-                          : dv.light_inline ? occupancy_grid(k_shade<FUSE_NEXT, false, SPEC_ONE_LIGHT>, s->sm_count, 0)
-                                          : occupancy_grid(k_shade<FUSE_NEXT, false, SPEC_FEW_LIGHTS>, s->sm_count, 0);
     s->grid_accumulate = occupancy_grid(k_accumulate, s->sm_count, 0);
-    if (s->mesh && !s->smallpt) {
-        s->mesh_box_scene = s->inline_area_light && dv.planes_grouped && dv.others_inline;
-        const size_t msm = mesh_smem(s);
-        s->grid_mesh = s->mesh_box_scene ? occupancy_grid(k_extend_mesh<false, SPEC_BOX_SCENE>, s->sm_count, msm) : occupancy_grid(k_extend_mesh<false>, s->sm_count, msm);
-        s->grid_mesh_last = s->mesh_box_scene ? occupancy_grid(k_extend_mesh<true, SPEC_BOX_SCENE>, s->sm_count, msm) : occupancy_grid(k_extend_mesh<true>, s->sm_count, msm);
+    s->shade = entry(smallpt ? k_shade<FUSE_NONE, true> : k_shade<FUSE_NONE, false>, 0);
+    s->shade_next = entry(fused_shade<FUSE_NEXT>(s->shade_spec), 0);
+    s->shade_last = entry(fused_shade<FUSE_LAST>(s->shade_spec), 0);
+    if (persistent_mesh) {
+        // persistent warps that refill idle lanes from the ray queue (ipt_trace.cuh), always in exact arithmetic
+        const bool box = s->mesh_spec == SPEC_BOX_SCENE;
+        s->extend[0][0] = s->extend[0][1] = entry(box ? k_extend_mesh<false, SPEC_BOX_SCENE> : k_extend_mesh<false>, IPT_MESH_SMEM_BYTES);
+        s->extend[1][0] = s->extend[1][1] = entry(box ? k_extend_mesh<true, SPEC_BOX_SCENE> : k_extend_mesh<true>, IPT_MESH_SMEM_BYTES);
+    } else {
+        const size_t sm = stack_smem(s);
+        with_scene_kind(s, [&](auto sp, auto ms) {
+            s->extend[0][1] = entry(k_extend<sp, ms, false, true>, sm);
+            s->extend[1][1] = entry(k_extend<sp, ms, true, true>, sm);
+            // SmallPt scenes with a mesh trace every depth in exact arithmetic: k_extend has no contracted mesh form
+            s->extend[0][0] = ms ? s->extend[0][1] : entry(k_extend<sp, false, false, false>, sm);
+            s->extend[1][0] = ms ? s->extend[1][1] : entry(k_extend<sp, false, true, false>, sm);
+        });
     }
-#define OCC(SP, MS)                                                                          \
-    s->grid_extend = occupancy_grid(k_extend<SP, MS, false>, s->sm_count, sm);               \
-    s->grid_extend_last = occupancy_grid(k_extend<SP, MS, true>, s->sm_count, sm)
-    DISPATCH_SM(s, OCC);
-#undef OCC
     guard.s = nullptr;
     *out = s;
     return IPT_OK;
@@ -691,11 +706,7 @@ int ipt_scene_destroy(ipt_scene* s) {
     cudaSetDevice(s->device);
     if (s->stream) cudaStreamSynchronize(s->stream);
     if (s->host_plane) ipt_plane_destroy(s->host_plane);
-    if (s->stream2) cudaStreamSynchronize(s->stream2);
     free_workspace(s->ws);
-    free_workspace(s->ws2);
-    if (s->stream2) cudaStreamDestroy(s->stream2);
-    if (s->ev_join) cudaEventDestroy(s->ev_join);
     lbvh_free(s->bvh);
     lbvh_free(s->light_bvh);
     cudaFree(s->d_prims); cudaFree(s->d_lights); cudaFree(s->d_light_cdf); cudaFree(s->d_light_guide); cudaFree(s->d_light_samp); cudaFree(s->d_mats); cudaFree(s->d_cnt); cudaFree(s->d_stats);
@@ -719,18 +730,10 @@ int ipt_scene_set_camera(ipt_scene* s, const ipt_camera* camera) {
 int ipt_scene_dispatch(ipt_scene* s, uint32_t out[IPT_DISPATCH_WORDS]) {
     if (!s || !out) return fail(IPT_ERR_INVALID, "null argument");
     std::lock_guard<std::recursive_mutex> lock__(s->mu);
-    // the same chain of predicates as the fused k_shade launches of ipt_render
-    const SceneSpec spec = s->smallpt ? SPEC_RUNTIME
-                           : s->dev.n_light_bvh ? SPEC_LIGHT_BVH
-                           : (s->inline_area_light && s->geom_fast && s->all_lambert) ? SPEC_LAMBERT_BOX
-                           : (s->inline_area_light && s->geom_fast) ? SPEC_BOX_SCENE
-                           : s->inline_area_light ? SPEC_ONE_AREA_LIGHT
-                           : s->dev.light_inline ? SPEC_ONE_LIGHT
-                                                 : SPEC_FEW_LIGHTS;
-    out[0] = (uint32_t)spec;
+    out[0] = (uint32_t)s->shade_spec;
     out[1] = s->smallpt;
     out[2] = s->mesh;
-    out[3] = s->mesh_box_scene;
+    out[3] = s->mesh_spec == SPEC_BOX_SCENE;
     out[4] = s->dev.lights_inside_box;
     out[5] = s->dev.light_inline;
     out[6] = s->dev.n_light_bvh;
@@ -751,9 +754,9 @@ int ipt_trace_batch(ipt_scene* s, const float* origins, const float* directions,
     CUDA_TRY(cudaMemcpyAsync(d_o.p, origins, 12 * n, cudaMemcpyHostToDevice, s->stream));
     CUDA_TRY(cudaMemcpyAsync(d_d.p, directions, 12 * n, cudaMemcpyHostToDevice, s->stream));
     unsigned blocks = (unsigned)((n + IPT_BLOCK - 1) / IPT_BLOCK);
-#define CALL(SP, MS) k_trace_batch<SP, MS><<<blocks, IPT_BLOCK, stack_smem(s), s->stream>>>(s->dev, d_o.p, d_d.p, n, d_prim.p, d_t.p, d_light.p, d_lp.p, d_out.p)
-    DISPATCH_SM(s, CALL);
-#undef CALL
+    with_scene_kind(s, [&](auto sp, auto ms) {
+        k_trace_batch<sp, ms><<<blocks, IPT_BLOCK, stack_smem(s), s->stream>>>(s->dev, d_o.p, d_d.p, n, d_prim.p, d_t.p, d_light.p, d_lp.p, d_out.p);
+    });
     CUDA_TRY(cudaGetLastError());
     if (prim_id) CUDA_TRY(cudaMemcpyAsync(prim_id, d_prim.p, 4 * n, cudaMemcpyDeviceToHost, s->stream));
     if (t) CUDA_TRY(cudaMemcpyAsync(t, d_t.p, 4 * n, cudaMemcpyDeviceToHost, s->stream));
@@ -774,9 +777,9 @@ int ipt_preview_batch(ipt_scene* s, const float* origins, const float* direction
     CUDA_TRY(cudaMemcpyAsync(d_o.p, origins, 12 * n, cudaMemcpyHostToDevice, s->stream));
     CUDA_TRY(cudaMemcpyAsync(d_d.p, directions, 12 * n, cudaMemcpyHostToDevice, s->stream));
     unsigned blocks = (unsigned)((n + IPT_BLOCK - 1) / IPT_BLOCK);
-#define CALL(SP, MS) k_preview_batch<SP, MS><<<blocks, IPT_BLOCK, stack_smem(s), s->stream>>>(s->dev, d_o.p, d_d.p, n, d_v.p)
-    DISPATCH_SM(s, CALL);
-#undef CALL
+    with_scene_kind(s, [&](auto sp, auto ms) {
+        k_preview_batch<sp, ms><<<blocks, IPT_BLOCK, stack_smem(s), s->stream>>>(s->dev, d_o.p, d_d.p, n, d_v.p);
+    });
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaMemcpyAsync(value, d_v.p, 4 * n, cudaMemcpyDeviceToHost, s->stream));
     CUDA_TRY(cudaStreamSynchronize(s->stream));
@@ -841,9 +844,9 @@ int ipt_mix_sample(ipt_scene* s, const float origin[3], const float direction[3]
     CUDA_TRY(d_w.alloc(3 * n)); CUDA_TRY(d_m.alloc(n)); CUDA_TRY(d_s.alloc(n)); CUDA_TRY(d_flag.alloc(1));
     f3 o{origin[0], origin[1], origin[2]}, d{direction[0], direction[1], direction[2]};
     unsigned blocks = (unsigned)((n + IPT_BLOCK - 1) / IPT_BLOCK);
-#define CALL(SP, MS) k_mix_sample<SP, MS><<<blocks, IPT_BLOCK, stack_smem(s), s->stream>>>(s->dev, o, d, (uint32_t)seed, (uint32_t)(seed >> 32), n, d_w.p, d_m.p, d_s.p, d_flag.p)
-    DISPATCH_SM(s, CALL);
-#undef CALL
+    with_scene_kind(s, [&](auto sp, auto ms) {
+        k_mix_sample<sp, ms><<<blocks, IPT_BLOCK, stack_smem(s), s->stream>>>(s->dev, o, d, (uint32_t)seed, (uint32_t)(seed >> 32), n, d_w.p, d_m.p, d_s.p, d_flag.p);
+    });
     CUDA_TRY(cudaGetLastError());
     int flag = 0;
     CUDA_TRY(cudaMemcpyAsync(&flag, d_flag.p, 4, cudaMemcpyDeviceToHost, s->stream));
@@ -1145,10 +1148,10 @@ static size_t workspace_bytes(size_t ray_cap, size_t hit_cap, size_t path_cap, b
     return 36 * ray_cap + 32 * std::max<size_t>(hit_cap, 1) * (two_hit_sets ? 2 : 1) + 4 * path_cap;
 }
 // IPT_OK, IPT_ERR_OVERFLOW when the device cannot hold this workspace (the caller retries with a smaller batch), or an error
-static int ensure_workspace(ipt_scene* s, Workspace& w, size_t ray_cap, size_t hit_cap, size_t path_cap, bool two_hit_sets) {
+static int ensure_workspace(ipt_scene* s, size_t ray_cap, size_t hit_cap, size_t path_cap, bool two_hit_sets) {
+    Workspace& w = s->ws;
     if (w.ray_cap >= ray_cap && w.hit_cap >= hit_cap && w.path_cap >= path_cap && (w.two_hit_sets || !two_hit_sets)) return IPT_OK;
     CUDA_TRY(cudaStreamSynchronize(s->stream));
-    CUDA_TRY(cudaStreamSynchronize(s->stream2));
     free_workspace(w);
     void** slots[8] = {(void**)&w.ray_o, (void**)&w.ray_d, (void**)&w.ray_x, (void**)&w.hit_a, (void**)&w.hit_b, (void**)&w.pathval, (void**)&w.hit_a2, (void**)&w.hit_b2};
     const size_t bytes[8] = {16 * ray_cap, 16 * ray_cap, 4 * ray_cap, 16 * std::max<size_t>(hit_cap, 1), 16 * std::max<size_t>(hit_cap, 1), 4 * path_cap,
@@ -1163,6 +1166,59 @@ static int ensure_workspace(ipt_scene* s, Workspace& w, size_t ray_cap, size_t h
         if (e != cudaSuccess) { free_workspace(w); return fail(IPT_ERR_CUDA, std::string("cudaMalloc (workspace): ") + cudaGetErrorString(e)); }
     }
     w.ray_cap = ray_cap; w.hit_cap = hit_cap; w.path_cap = path_cap; w.two_hit_sets = two_hit_sets;
+    return IPT_OK;
+}
+
+// The paths per batch of a render (`requested`, or a default from the widest tree levels), and the scene's workspace
+// grown to hold the queues of one batch
+static int size_batch(ipt_scene* s, uint64_t requested, uint64_t total_paths, uint64_t tile_pixels, uint64_t max_ray_w,
+                      uint64_t max_queued_w, uint64_t max_hit_w, uint32_t slot_bits, bool fuse_next, uint64_t& batch) {
+    // default batch: as many paths as keep the widest tree level near 2^28 rays (2^19 paths at 16/8/4/2; up to 2^23
+    // for narrow schedules such as depth 8 with one child per hit, whose deeper levels would otherwise be tiny launches)
+    // (with the fused last level the widest level is not queued: 2^27 / widest queued level, i.e. 2^20 paths at 16/8/4/2)
+    // (fused shade kernels: what is queued are the hits, 2^28 / widest hit level = 2^21 paths at 16/8/4/2, 17 GB of
+    // hit records in the two sets; 2^20 paths is 1.5 % slower, 2^22 0.3 % faster)
+    uint64_t batch_rays = (max_queued_w < max_ray_w && !fuse_next) ? (1ull << 27) : (1ull << 28);
+    uint64_t batch_w = fuse_next ? max_hit_w : max_queued_w;
+    // (narrow schedules such as depth 8 with one child per hit: up to 2^25 paths. Every launch of the persistent mesh kernel
+    // ends with its longest ray — ~1000 dependent node visits walked by a single lane, ~0.9 ms whatever the launch holds —
+    // so eight launches per batch want as many rays per launch as memory allows: 2^23 / 2^24 / 2^25 paths per batch give
+    // C3 325 / 369 / 376 and C4 290 / 322 / 332 Mpaths/s; 2^25 paths are 2.4 GB of queues)
+    batch = requested ? requested : std::min<uint64_t>(1ull << 25, std::max<uint64_t>(1ull << 16, batch_rays / batch_w));
+    batch = std::min<uint64_t>(batch, slot_bits >= 32 ? 0xFFFFFFFFull : (1ull << slot_bits));
+    // Queue memory is sized for the worst case of a batch (no overflow path). Budget: IPT_QUEUE_BUDGET_GB (default 24 GiB:
+    // 2^21 paths at 16/8/4/2 need 2 x 8.6 GB of hit records; halving the batch costs ~1.5 %, profiles/tuning_r02.md), never
+    // more than 80 % of what the device has free right now (plus what this scene's workspace already holds), and the
+    // batch is halved again whenever the allocation itself fails.
+    uint64_t budget = 24ull << 30;
+    if (const char* e = std::getenv("IPT_QUEUE_BUDGET_GB")) { double gb = std::atof(e); if (gb > 0) budget = (uint64_t)(gb * (double)(1ull << 30)); }
+    Workspace& ws = s->ws;
+    const uint64_t choice_key[5] = {batch, max_queued_w, max_hit_w, budget, fuse_next ? 1ull : 0ull};
+    if (ws.choice_batch && ws.path_cap && std::memcmp(choice_key, ws.choice_key, sizeof choice_key) == 0) {
+        batch = ws.choice_batch; // same question as last time, and a workspace it led to is still allocated
+    } else {
+        size_t free_b = 0, total_b = 0;
+        if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess) {
+            uint64_t held = ws.path_cap ? workspace_bytes(ws.ray_cap, ws.hit_cap, ws.path_cap, ws.two_hit_sets) : 0;
+            budget = std::min<uint64_t>(budget, (uint64_t)((double)(free_b + held) * 0.8));
+        } else cudaGetLastError();
+        while (batch > 1024 && workspace_bytes(batch * max_queued_w, batch * max_hit_w, batch, fuse_next) > budget) batch >>= 1;
+    }
+    const uint64_t batch_unclamped = batch;
+    batch = std::max<uint64_t>(1, std::min<uint64_t>(batch, std::max<uint64_t>(total_paths, 1)));
+    if (tile_pixels + batch > 0xFFFFFFFFull) return fail(IPT_ERR_UNSUPPORTED, "tile too large: tile pixels + batch must stay below 2^32");
+    bool alloc_halved = false;
+    for (;;) {
+        int rc = ensure_workspace(s, batch * max_queued_w, batch * max_hit_w, batch, fuse_next);
+        if (rc == IPT_OK) break;
+        if (rc != IPT_ERR_OVERFLOW || batch <= 1024) return rc;
+        batch >>= 1; // another tenant (torch, NCCL) took the memory between the query and the allocation
+        alloc_halved = true;
+    }
+    if (!alloc_halved) {
+        std::memcpy(ws.choice_key, choice_key, sizeof choice_key);
+        ws.choice_batch = batch_unclamped;
+    }
     return IPT_OK;
 }
 
@@ -1207,72 +1263,20 @@ int ipt_render(ipt_scene* s, ipt_plane* plane, const ipt_render_params* p, ipt_r
     while ((1ull << idx_bits) < max_ray_w) ++idx_bits;
     uint32_t slot_bits = 32 - idx_bits;
     uint64_t total_paths = (uint64_t)tw * th * p->pass_count;
-    // default batch: as many paths as keep the widest tree level near 2^28 rays (2^19 paths at 16/8/4/2; up to 2^23
-    // for narrow schedules such as depth 8 with one child per hit, whose deeper levels would otherwise be tiny launches)
-    // (with the fused last level the widest level is not queued: 2^27 / widest queued level, i.e. 2^20 paths at 16/8/4/2)
-    // (fused shade kernels: what is queued are the hits, 2^28 / widest hit level = 2^21 paths at 16/8/4/2, 17 GB of
-    // hit records in the two sets; 2^20 paths is 1.5 % slower, 2^22 0.3 % faster)
-    uint64_t batch_rays = (max_queued_w < max_ray_w && !fuse_next) ? (1ull << 27) : (1ull << 28);
-    uint64_t batch_w = fuse_next ? max_hit_w : max_queued_w;
-    // (narrow schedules such as depth 8 with one child per hit: up to 2^25 paths. Every launch of the persistent mesh kernel
-    // ends with its longest ray — ~1000 dependent node visits walked by a single lane, ~0.9 ms whatever the launch holds —
-    // so eight launches per batch want as many rays per launch as memory allows: 2^23 / 2^24 / 2^25 paths per batch give
-    // C3 325 / 369 / 376 and C4 290 / 322 / 332 Mpaths/s; 2^25 paths are 2.4 GB of queues)
-    uint64_t batch = p->batch_paths ? p->batch_paths : std::min<uint64_t>(1ull << 25, std::max<uint64_t>(1ull << 16, batch_rays / batch_w));
-    batch = std::min<uint64_t>(batch, slot_bits >= 32 ? 0xFFFFFFFFull : (1ull << slot_bits));
-    // Queue memory is sized for the worst case of a batch (no overflow path). Budget: IPT_QUEUE_BUDGET_GB (default 24 GiB:
-    // 2^21 paths at 16/8/4/2 need 2 x 8.6 GB of hit records; halving the batch costs ~1.5 %, profiles/tuning_r02.md), never
-    // more than 80 % of what the device has free right now (plus what this scene's workspace already holds), and the
-    // batch is halved again whenever the allocation itself fails.
-    uint64_t budget = 24ull << 30;
-    if (const char* e = std::getenv("IPT_QUEUE_BUDGET_GB")) { double gb = std::atof(e); if (gb > 0) budget = (uint64_t)(gb * (double)(1ull << 30)); }
-    const uint64_t choice_key[5] = {batch, max_queued_w, max_hit_w, budget, fuse_next ? 1ull : 0ull};
-    if (s->ws.choice_batch && s->ws.path_cap && std::memcmp(choice_key, s->ws.choice_key, sizeof choice_key) == 0) {
-        batch = s->ws.choice_batch; // same question as last time, and a workspace it led to is still allocated
-    } else {
-        size_t free_b = 0, total_b = 0;
-        if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess) {
-            const Workspace& w0 = s->ws;
-            uint64_t held = w0.path_cap ? workspace_bytes(w0.ray_cap, w0.hit_cap, w0.path_cap, w0.two_hit_sets) : 0;
-            budget = std::min<uint64_t>(budget, (uint64_t)((double)(free_b + held) * 0.8));
-        } else cudaGetLastError();
-        while (batch > 1024 && workspace_bytes(batch * max_queued_w, batch * max_hit_w, batch, fuse_next) > budget) batch >>= 1;
-    }
-    const uint64_t batch_unclamped = batch;
-    batch = std::max<uint64_t>(1, std::min<uint64_t>(batch, std::max<uint64_t>(total_paths, 1)));
-    // Mesh scenes keep TWO batches in flight, each on its own stream with its own queues (IPT_RENDER_LANES): a launch of the
-    // persistent traversal kernel ends with a tail — its longest rays, walked by a few lanes — during which the blocks of
-    // the other batch's launch move onto the idle SMs. A job that would fit one batch is split in two for that.
-    const bool two_lanes = IPT_RENDER_LANES == 2 && s->mesh && !s->smallpt && total_paths >= (1ull << 21);
-    if (two_lanes) batch = std::min<uint64_t>(batch, (total_paths + 1) / 2);
-    if ((uint64_t)tw * th + batch > 0xFFFFFFFFull) return fail(IPT_ERR_UNSUPPORTED, "tile too large: tile pixels + batch must stay below 2^32");
-    bool alloc_halved = false;
-    for (;;) {
-        int rc = ensure_workspace(s, s->ws, batch * max_queued_w, batch * max_hit_w, batch, fuse_next);
-        if (rc == IPT_OK && two_lanes) rc = ensure_workspace(s, s->ws2, batch * max_queued_w, batch * max_hit_w, batch, fuse_next);
-        if (rc == IPT_OK) break;
-        if (rc != IPT_ERR_OVERFLOW || batch <= 1024) return rc;
-        batch >>= 1; // another tenant (torch, NCCL) took the memory between the query and the allocation
-        alloc_halved = true;
-    }
-    if (!alloc_halved) {
-        std::memcpy(s->ws.choice_key, choice_key, sizeof choice_key);
-        s->ws.choice_batch = batch_unclamped;
-    }
+    uint64_t batch = 0;
+    int rc = size_batch(s, p->batch_paths, total_paths, (uint64_t)tw * th, max_ray_w, max_queued_w, max_hit_w, slot_bits, fuse_next, batch);
+    if (rc) return rc;
 
+    const Workspace& W = s->ws;
     RenderCtx C;
     std::memset(&C, 0, sizeof C);
-    auto use_lane = [&](int lane) { // the queues and counters of one lane
-        const Workspace& W = lane ? s->ws2 : s->ws;
-        C.ray_o = W.ray_o; C.ray_d = W.ray_d; C.ray_x = W.ray_x; C.pathval = W.pathval;
-        C.hit_a[0] = W.hit_a; C.hit_b[0] = W.hit_b;
-        C.hit_a[1] = fuse_next ? W.hit_a2 : W.hit_a; C.hit_b[1] = fuse_next ? W.hit_b2 : W.hit_b;
-        C.cnt = s->d_cnt + (size_t)lane * IPT_CNT_WORDS; C.fetch = C.cnt + (2 * IPT_MAX_DEPTH + 2);
-    };
-    use_lane(0);
+    C.ray_o = W.ray_o; C.ray_d = W.ray_d; C.ray_x = W.ray_x; C.pathval = W.pathval;
+    C.hit_a[0] = W.hit_a; C.hit_b[0] = W.hit_b;
+    C.hit_a[1] = fuse_next ? W.hit_a2 : W.hit_a; C.hit_b[1] = fuse_next ? W.hit_b2 : W.hit_b;
+    C.cnt = s->d_cnt; C.fetch = C.cnt + (2 * IPT_MAX_DEPTH + 2);
     C.stats = s->d_stats;
     C.sum = plane->sum; C.sumsq = plane->sumsq; C.count = plane->count;
-    C.ray_cap = (uint32_t)std::min<size_t>(s->ws.ray_cap, 0xFFFFFFFFull); C.hit_cap = (uint32_t)std::min<size_t>(s->ws.hit_cap, 0xFFFFFFFFull);
+    C.ray_cap = (uint32_t)std::min<size_t>(W.ray_cap, 0xFFFFFFFFull); C.hit_cap = (uint32_t)std::min<size_t>(W.hit_cap, 0xFFFFFFFFull);
     C.width = p->width; C.height = p->height;
     C.tile_x0 = tx0; C.tile_y0 = ty0; C.tile_w = tw; C.tile_h = th; C.tile_pixels = tw * th;
     C.pass_begin = p->pass_begin;
@@ -1285,6 +1289,7 @@ int ipt_render(ipt_scene* s, ipt_plane* plane, const ipt_render_params* p, ipt_r
     C.div_tile_w = make_fastdiv(C.tile_w);
     C.plane_mode = p->plane_mode; C.flags = p->flags;
 
+    const cudaStream_t st = s->stream;
     const bool timing = (p->flags & IPT_FLAG_TIME_KERNELS) != 0;
     bool timing_failed = false;
     std::vector<int> ev_kind; // 0 generate 1 extend 2 shade 3 accumulate, one entry per bracketed launch
@@ -1298,112 +1303,60 @@ int ipt_render(ipt_scene* s, ipt_plane* plane, const ipt_render_params* p, ipt_r
         return s->events[ev_used++];
     };
     uint32_t launches = 0;
-    CUDA_TRY(cudaMemsetAsync(s->d_stats, 0, sizeof(unsigned long long) * ST_COUNT, s->stream));
-    CUDA_TRY(cudaEventRecord(s->ev_begin, s->stream));
-    if (two_lanes) CUDA_TRY(cudaStreamWaitEvent(s->stream2, s->ev_begin, 0));
-    size_t sm = stack_smem(s);
-    const size_t msm = mesh_smem(s);
+    auto timed = [&](int kind, auto&& launch) { // one launch, bracketed by events when the kernels are timed
+        if (timing) cudaEventRecord(ev_next(), st);
+        launch();
+        ++launches;
+        if (timing) { cudaEventRecord(ev_next(), st); ev_kind.push_back(kind); }
+    };
+    // a kernel of the scene's table at depth d, never with more blocks than the level has rays for
+    auto run = [&](const RenderKernel& k, int kind, uint32_t d, int cap_blocks) {
+        timed(kind, [&] { k.kernel<<<std::max(1, std::min(k.grid, cap_blocks)), IPT_BLOCK, k.smem, st>>>(s->dev, C, d); });
+    };
+    CUDA_TRY(cudaMemsetAsync(s->d_stats, 0, sizeof(unsigned long long) * ST_COUNT, st));
+    CUDA_TRY(cudaEventRecord(s->ev_begin, st));
     uint32_t batches = 0;
     for (uint64_t g0 = 0; g0 < total_paths; g0 += batch, ++batches) {
-        const int lane = two_lanes ? (int)(batches & 1u) : 0;
-        cudaStream_t st = lane ? s->stream2 : s->stream;
-        use_lane(lane);
         C.g0 = g0;
         C.pass0 = p->pass_begin + (uint32_t)(g0 / C.tile_pixels);
         C.rem0 = (uint32_t)(g0 % C.tile_pixels);
         C.batch = (uint32_t)std::min<uint64_t>(batch, total_paths - g0);
         CUDA_TRY(cudaMemsetAsync(C.cnt, 0, sizeof(uint32_t) * IPT_CNT_WORDS, st));
-#define TIMED(kind, LAUNCH)                                             \
-    do {                                                                \
-        if (timing) { cudaEventRecord(ev_next(), st); }         \
-        LAUNCH;                                                         \
-        ++launches;                                                     \
-        if (timing) { cudaEventRecord(ev_next(), st); ev_kind.push_back(kind); } \
-    } while (0)
         int gg = std::min<int>(s->grid_generate, (int)((C.batch + IPT_BLOCK - 1) / IPT_BLOCK));
-        TIMED(0, (k_generate<<<gg, IPT_BLOCK, 0, st>>>(s->dev, C)));
+        timed(0, [&] { k_generate<<<gg, IPT_BLOCK, 0, st>>>(s->dev, C); });
         bool traced = false; // the shade kernel of the previous depth has already traced the rays of this depth
         for (uint32_t d = 0; d < p->depth_max; ++d) {
             if (width_at[d] == 0) break;
             bool last = (d + 1 == p->depth_max) || p->schedule[d] == 0;
-            // never launch more warps than the level can have rays
             uint64_t max_rays = (uint64_t)C.batch * width_at[d];
             int cap_blocks = (int)std::min<uint64_t>((max_rays + IPT_BLOCK - 1) / IPT_BLOCK, 1u << 30);
-            const bool persistent_mesh = s->mesh && !s->smallpt;
-            if (persistent_mesh) {
-                // mesh scenes: persistent warps that refill idle lanes from the ray queue (ipt_trace.cuh)
-                if (last) {
-                    if (s->mesh_box_scene) TIMED(1, (k_extend_mesh<true, SPEC_BOX_SCENE><<<std::max(1, std::min(s->grid_mesh_last, cap_blocks)), IPT_BLOCK, msm, st>>>(s->dev, C, d)));
-                    else TIMED(1, (k_extend_mesh<true><<<std::max(1, std::min(s->grid_mesh_last, cap_blocks)), IPT_BLOCK, msm, st>>>(s->dev, C, d)));
-                    break;
-                }
-                if (s->mesh_box_scene) TIMED(1, (k_extend_mesh<false, SPEC_BOX_SCENE><<<std::max(1, std::min(s->grid_mesh, cap_blocks)), IPT_BLOCK, msm, st>>>(s->dev, C, d)));
-                else TIMED(1, (k_extend_mesh<false><<<std::max(1, std::min(s->grid_mesh, cap_blocks)), IPT_BLOCK, msm, st>>>(s->dev, C, d)));
-                int gs2 = std::max(1, std::min(s->grid_shade, cap_blocks));
-                TIMED(2, (k_shade<FUSE_NONE, false><<<gs2, IPT_BLOCK, 0, st>>>(s->dev, C, d)));
-                continue;
-            }
             // camera rays are traced with the reference's exact arithmetic; rays downstream of a random number with the
             // contracted form the fused shade kernels use too (so fused and queued runs agree ray for ray)
             const bool exact_d = d == 0 || !IPT_FAST_SECONDARY;
             if (!traced) { // the rays of this depth wait in the ray queue (depth 0, or an unfused run)
-                if (last) {
-                    int g = std::max(1, std::min(s->grid_extend_last, cap_blocks));
-#define CALL(SP, MS)                                                                                             \
-    if (MS || exact_d) TIMED(1, (k_extend<SP, MS, true, true><<<g, IPT_BLOCK, sm, st>>>(s->dev, C, d))); \
-    else TIMED(1, (k_extend<SP, false, true, false><<<g, IPT_BLOCK, sm, st>>>(s->dev, C, d)))
-                    DISPATCH_SM(s, CALL);
-#undef CALL
-                    break;
-                }
-                int g = std::max(1, std::min(s->grid_extend, cap_blocks));
-#define CALL(SP, MS)                                                                                              \
-    if (MS || exact_d) TIMED(1, (k_extend<SP, MS, false, true><<<g, IPT_BLOCK, sm, st>>>(s->dev, C, d))); \
-    else TIMED(1, (k_extend<SP, false, false, false><<<g, IPT_BLOCK, sm, st>>>(s->dev, C, d)))
-                DISPATCH_SM(s, CALL);
-#undef CALL
+                run(s->extend[last][exact_d], 1, d, cap_blocks);
+                if (last) break;
             }
             traced = false;
             // the children of this level are the last traced depth: resolve them inside the shade kernel (no queue, no
             // k_extend<LAST> launch); analytic scenes only, and not when a flag asks for the unfused behaviour
             bool child_last = width_at[d + 1] != 0 && ((d + 2 == p->depth_max) || p->schedule[d + 1] == 0);
             if (child_last && fuse_last) {
-                int gf = std::max(1, std::min(s->grid_shade_fused, cap_blocks));
-                if (s->smallpt) TIMED(2, (k_shade<FUSE_LAST, true><<<gf, IPT_BLOCK, 0, st>>>(s->dev, C, d)));
-                else if (s->dev.n_light_bvh) TIMED(2, (k_shade<FUSE_LAST, false, SPEC_LIGHT_BVH><<<gf, IPT_BLOCK, 0, st>>>(s->dev, C, d)));
-                else if (s->inline_area_light && s->geom_fast && s->all_lambert) TIMED(2, (k_shade<FUSE_LAST, false, SPEC_LAMBERT_BOX><<<gf, IPT_BLOCK, 0, st>>>(s->dev, C, d)));
-                else if (s->inline_area_light && s->geom_fast) TIMED(2, (k_shade<FUSE_LAST, false, SPEC_BOX_SCENE><<<gf, IPT_BLOCK, 0, st>>>(s->dev, C, d)));
-                else if (s->inline_area_light) TIMED(2, (k_shade<FUSE_LAST, false, SPEC_ONE_AREA_LIGHT><<<gf, IPT_BLOCK, 0, st>>>(s->dev, C, d)));
-                else if (s->dev.light_inline) TIMED(2, (k_shade<FUSE_LAST, false, SPEC_ONE_LIGHT><<<gf, IPT_BLOCK, 0, st>>>(s->dev, C, d)));
-                else TIMED(2, (k_shade<FUSE_LAST, false, SPEC_FEW_LIGHTS><<<gf, IPT_BLOCK, 0, st>>>(s->dev, C, d)));
+                run(s->shade_last, 2, d, cap_blocks);
                 break;
             }
             if (fuse_next && width_at[d + 1] != 0) {
-                int gn = std::max(1, std::min(s->grid_shade_next, cap_blocks));
-                if (s->smallpt) TIMED(2, (k_shade<FUSE_NEXT, true><<<gn, IPT_BLOCK, 0, st>>>(s->dev, C, d)));
-                else if (s->dev.n_light_bvh) TIMED(2, (k_shade<FUSE_NEXT, false, SPEC_LIGHT_BVH><<<gn, IPT_BLOCK, 0, st>>>(s->dev, C, d)));
-                else if (s->inline_area_light && s->geom_fast && s->all_lambert) TIMED(2, (k_shade<FUSE_NEXT, false, SPEC_LAMBERT_BOX><<<gn, IPT_BLOCK, 0, st>>>(s->dev, C, d)));
-                else if (s->inline_area_light && s->geom_fast) TIMED(2, (k_shade<FUSE_NEXT, false, SPEC_BOX_SCENE><<<gn, IPT_BLOCK, 0, st>>>(s->dev, C, d)));
-                else if (s->inline_area_light) TIMED(2, (k_shade<FUSE_NEXT, false, SPEC_ONE_AREA_LIGHT><<<gn, IPT_BLOCK, 0, st>>>(s->dev, C, d)));
-                else if (s->dev.light_inline) TIMED(2, (k_shade<FUSE_NEXT, false, SPEC_ONE_LIGHT><<<gn, IPT_BLOCK, 0, st>>>(s->dev, C, d)));
-                else TIMED(2, (k_shade<FUSE_NEXT, false, SPEC_FEW_LIGHTS><<<gn, IPT_BLOCK, 0, st>>>(s->dev, C, d)));
+                run(s->shade_next, 2, d, cap_blocks);
                 traced = true; // the rays of depth d+1 are traced by this launch: no k_extend for them
                 continue;
             }
-            int gs = std::max(1, std::min(s->grid_shade, cap_blocks));
-            if (s->smallpt) TIMED(2, (k_shade<FUSE_NONE, true><<<gs, IPT_BLOCK, 0, st>>>(s->dev, C, d))); // reference-order sampling (ipt_shading.cuh)
-            else TIMED(2, (k_shade<FUSE_NONE, false><<<gs, IPT_BLOCK, 0, st>>>(s->dev, C, d)));
+            run(s->shade, 2, d, cap_blocks);
         }
-        TIMED(3, (k_accumulate<<<std::max(1, gg), IPT_BLOCK, 0, st>>>(C)));
-#undef TIMED
+        timed(3, [&] { k_accumulate<<<std::max(1, gg), IPT_BLOCK, 0, st>>>(C); });
         CUDA_TRY(cudaGetLastError());
     }
-    if (two_lanes) {
-        CUDA_TRY(cudaEventRecord(s->ev_join, s->stream2));
-        CUDA_TRY(cudaStreamWaitEvent(s->stream, s->ev_join, 0));
-    }
-    CUDA_TRY(cudaEventRecord(s->ev_end, s->stream));
-    CUDA_TRY(cudaStreamSynchronize(s->stream));
+    CUDA_TRY(cudaEventRecord(s->ev_end, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
     CUDA_TRY(cudaGetLastError());
 
 #ifdef IPT_DEBUG_BOUNDS

@@ -17,7 +17,6 @@ VARIANTS = {
     "lightq": ["IPT_LIGHT_QNODES=1"],      # light LBVH through its 32-byte quantised nodes (measured: no gain)
     "nosamp": ["IPT_LIGHT_SAMP_RECORDS=0"], # light sampling from the 112-byte records
     "walls": ["IPT_SHADOW_SKIP_WALLS=0"],  # shadow rays of box scenes test the wall planes too
-    "twolanes": ["IPT_RENDER_LANES=2"],   # mesh scenes: two batches in flight on two streams (measured: +2-4 % at best)
     "m_s8": ["IPT_TRAV_STEPS=8"], "m_s32": ["IPT_TRAV_STEPS=32"], "m_l16": ["IPT_LEAF_BATCH=16"], "m_b5": ["IPT_MESH_MIN_BLOCKS=5"],
     "m_l4": ["IPT_LEAF_BATCH=4"], "m_l8": ["IPT_LEAF_BATCH=8"], "m_l10": ["IPT_LEAF_BATCH=10"], "m_r2": ["IPT_REFILL_MIN=2"], "m_r8": ["IPT_REFILL_MIN=8"], "m_v1": ["IPT_VISITS_PER_ROUND=1"],  # mesh kernel sweeps
     "m_st8": ["IPT_STACK_SHORT=8"], "m_st16": ["IPT_STACK_SHORT=16"], "m_st20": ["IPT_STACK_SHORT=20"], "m_st24": ["IPT_STACK_SHORT=24"], "m_st32": ["IPT_STACK_SHORT=32"], "m_b3": ["IPT_MESH_MIN_BLOCKS=3"], "m_s24": ["IPT_TRAV_STEPS=24"],
