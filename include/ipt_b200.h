@@ -209,6 +209,31 @@ int ipt_scene_set_camera(ipt_scene* scene, const ipt_camera* camera);
 #define IPT_DISPATCH_WORDS 7
 int ipt_scene_dispatch(ipt_scene* scene, uint32_t out[IPT_DISPATCH_WORDS]);
 
+/* Moving a mesh without recreating the scene (its stream, workspace and planes stay). */
+enum ipt_update_flags {
+    IPT_UPDATE_DEVICE_POINTER = 1u, /* `triangles` is device memory on the scene's device (e.g. a CUDA tensor) */
+    IPT_UPDATE_REBUILD = 2u         /* full LBVH build over the new vertices; default: refit the existing tree */
+};
+/* Replace the vertices of the scene's triangle mesh (9 floats per triangle, v0 e1 e2, as in ipt_scene_desc).
+ * n_triangles must equal the scene's count; a different count needs a new scene. Lights are not moved.
+ *   Result: afterwards every result (traces, renders, ipt_scene_dispatch) equals that of a scene created from the new
+ *     triangles. The exception is the tree itself after a refit: it keeps the topology, Morton keys and sorted order of
+ *     its last build and only recomputes every box, so its node boxes differ, and so do the node-visit counters of renders
+ *     (bvh_nodes_visited, triangles_tested). A refit is cheap; the tree's quality degrades as the mesh moves away from the
+ *     pose it was built in, and IPT_UPDATE_REBUILD restores it.
+ *   Synchronisation: takes the scene's mutex and runs on the scene's stream, after the work already enqueued there. It
+ *     returns once the update is complete: the caller may then free or overwrite its buffer. With
+ *     IPT_UPDATE_DEVICE_POINTER the caller must have finished writing the buffer on its own stream before the call; the
+ *     library waits on no other stream.
+ *   Planes made on the scene stay valid, and their accumulators are not touched: clearing them is the caller's decision,
+ *     as after ipt_scene_set_camera.
+ *   Errors (IPT_ERR_INVALID): a null argument, unknown flag bits, a scene without a mesh, a count that differs from the
+ *     scene's, and a pointer whose kind does not match the flag (by cudaPointerGetAttributes: with
+ *     IPT_UPDATE_DEVICE_POINTER it must be device or managed memory on the scene's device, without it it must not be
+ *     device memory), or that is not aligned to a float.
+ *   Atomicity: if an allocation fails (IPT_ERR_CUDA), the scene keeps its previous triangles and tree. */
+int ipt_scene_update_triangles(ipt_scene* scene, const float* triangles, uint64_t n_triangles, uint32_t flags);
+
 /* The reference's five scenes + this repo's benchmark scenes as descriptions:
  * "box" (make_scene_box, the default), "fractal", "smallpt", "square", "corner", "openspheres", "cornell" (C2),
  * "mixedlights" (one of every Light class over the default geometry),

@@ -21,6 +21,7 @@ IPT_ERR_NO_DEVICE = 3
 SPEC_FEW_LIGHTS, SPEC_LIGHT_BVH, SPEC_RUNTIME, SPEC_ONE_LIGHT, SPEC_ONE_AREA_LIGHT, SPEC_BOX_SCENE, SPEC_LAMBERT_BOX = range(7)
 DISPATCH_FIELDS = ("spec", "smallpt", "mesh", "mesh_box_scene", "lights_inside_box", "light_inline", "n_light_bvh")
 DISPATCH_WORDS = len(DISPATCH_FIELDS)
+UPDATE_DEVICE_POINTER, UPDATE_REBUILD = 1, 2  # ipt_update_flags
 
 import os
 
@@ -100,6 +101,7 @@ SIGNATURES = {
     "ipt_scene_destroy": (C.c_int, [_vp]),
     "ipt_scene_set_camera": (C.c_int, [_vp, C.POINTER(Camera)]),
     "ipt_scene_dispatch": (C.c_int, [_vp, u32p]),
+    "ipt_scene_update_triangles": (C.c_int, [_vp, _vp, C.c_uint64, C.c_uint32]),
     "ipt_sample_scene": (C.c_int, [C.c_char_p, C.POINTER(C.POINTER(SceneDesc))]),
     "ipt_scene_desc_free": (C.c_int, [C.POINTER(SceneDesc)]),
     "ipt_light_derived": (C.c_int, [C.POINTER(Light), f32p, f32p, f32p]),
@@ -265,6 +267,7 @@ class Scene:
 
     def __init__(self, description: SceneDescription, device: int = 0):
         self.description = description
+        self.device = device
         self.handle = _vp()
         check(load().ipt_scene_create(description.ptr, device, C.byref(self.handle)))
 
@@ -288,6 +291,33 @@ class Scene:
         out = np.zeros(DISPATCH_WORDS, np.uint32)
         check(load().ipt_scene_dispatch(self.handle, _ptr(out, u32p)))
         return dict(zip(DISPATCH_FIELDS, (int(v) for v in out)))
+
+    def update_triangles(self, triangles, rebuild: bool = False):
+        """ipt_scene_update_triangles: new vertices for the scene's mesh, same triangle count. `triangles` is a C-contiguous
+        float32 numpy array of shape (n, 9) or (9n,) (host input), or a contiguous float32 CUDA tensor of either shape on the
+        scene's device (device input: torch's current stream on that device is synchronised first). rebuild=False refits
+        the existing tree, rebuild=True builds it anew over the new vertices."""
+        flags = UPDATE_REBUILD if rebuild else 0
+        if isinstance(triangles, np.ndarray):
+            if triangles.dtype != np.float32 or not triangles.flags.c_contiguous:
+                raise TypeError("triangles: a C-contiguous float32 array is required")
+            shape, ptr = triangles.shape, triangles.ctypes.data
+        else:
+            import torch  # the only torch use of this module: device input
+
+            if not isinstance(triangles, torch.Tensor):
+                raise TypeError(f"triangles: a numpy array or a CUDA tensor is required, not {type(triangles).__name__}")
+            if triangles.dtype != torch.float32 or not triangles.is_contiguous():
+                raise TypeError("triangles: a contiguous float32 tensor is required")
+            if triangles.device.type != "cuda" or triangles.device.index != self.device:
+                raise ValueError(f"triangles: a tensor on cuda:{self.device} (the scene's device) is required, not on {triangles.device}")
+            torch.cuda.current_stream(triangles.device).synchronize()
+            shape, ptr = tuple(triangles.shape), triangles.data_ptr()
+            flags |= UPDATE_DEVICE_POINTER
+        if not (len(shape) == 2 and shape[1] == 9 or len(shape) == 1 and shape[0] % 9 == 0):
+            raise ValueError(f"triangles: shape (n, 9) or (9n,) required, got {shape}")
+        n = shape[0] if len(shape) == 2 else shape[0] // 9
+        check(load().ipt_scene_update_triangles(self.handle, ptr, n, flags))
 
     def trace_batch(self, origins, directions):
         o, d = _f32(origins).reshape(-1, 3), _f32(directions).reshape(-1, 3)

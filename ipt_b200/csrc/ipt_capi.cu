@@ -433,6 +433,15 @@ static RenderKernel::Fn fused_shade(SceneSpec spec) {
     }
 }
 
+// the device scene's view of the mesh LBVH
+static void bind_mesh(ipt_scene* s) {
+    s->dev.tris = s->bvh.tri_records;
+    s->dev.tri_id = s->bvh.sorted_ids;
+    s->dev.nodes = s->bvh.nodes;
+    s->dev.qnodes = s->bvh.qnodes;
+    s->dev.grid = s->bvh.grid;
+}
+
 static size_t stack_smem(const ipt_scene* s) { return s->mesh ? (size_t)IPT_STACK_SHORT * IPT_BLOCK * sizeof(uint32_t) : 0; }
 
 template <class T>
@@ -621,15 +630,11 @@ int ipt_scene_create(const ipt_scene_desc* desc, int device, ipt_scene** out) {
     for (const DevMaterial& m : mats) if (m.ddf != IPT_DDF_COSINE) all_lambert = false;
     if (s->mesh) {
         std::string err;
-        if (lbvh_build(desc->triangles, (uint32_t)desc->n_triangles, s->stream, s->bvh, err) != 0)
+        if (lbvh_build_host(desc->triangles, (uint32_t)desc->n_triangles, s->stream, s->bvh, err) != 0)
             return fail(IPT_ERR_CUDA, "LBVH build failed: " + err);
         dv.n_tris = (uint32_t)desc->n_triangles;
         dv.tri_material = desc->triangle_material;
-        dv.tris = s->bvh.tri_records;
-        dv.tri_id = s->bvh.sorted_ids;
-        dv.nodes = s->bvh.nodes;
-        dv.qnodes = s->bvh.qnodes;
-        dv.grid = s->bvh.grid;
+        bind_mesh(s);
     }
     // many area lights: LBVH over them (nearest-light and all-hits density queries instead of O(L) scans)
     {
@@ -647,7 +652,7 @@ int ipt_scene_create(const ipt_scene_desc* desc, int device, ipt_scene** out) {
                 extra[3 * (size_t)i + 2] = lights[i].weight;
             }
             std::string err;
-            if (lbvh_build(ltris.data(), desc->n_lights, s->stream, s->light_bvh, err, extra.data()) != 0)
+            if (lbvh_build_host(ltris.data(), desc->n_lights, s->stream, s->light_bvh, err, extra.data()) != 0)
                 return fail(IPT_ERR_CUDA, "light LBVH build failed: " + err);
             dv.light_nodes = s->light_bvh.nodes;
             dv.light_qnodes = s->light_bvh.qnodes;
@@ -737,6 +742,53 @@ int ipt_scene_dispatch(ipt_scene* s, uint32_t out[IPT_DISPATCH_WORDS]) {
     out[4] = s->dev.lights_inside_box;
     out[5] = s->dev.light_inline;
     out[6] = s->dev.n_light_bvh;
+    return IPT_OK;
+}
+
+int ipt_scene_update_triangles(ipt_scene* s, const float* triangles, uint64_t n_triangles, uint32_t flags) {
+    if (!s || !triangles) return fail(IPT_ERR_INVALID, "ipt_scene_update_triangles: null argument");
+    if (flags & ~(uint32_t)(IPT_UPDATE_DEVICE_POINTER | IPT_UPDATE_REBUILD))
+        return fail(IPT_ERR_INVALID, "ipt_scene_update_triangles: unknown flag bits " + std::to_string(flags));
+    std::lock_guard<std::recursive_mutex> lock__(s->mu);
+    if (!s->mesh) return fail(IPT_ERR_INVALID, "ipt_scene_update_triangles: the scene has no triangle mesh");
+    if (n_triangles != s->bvh.n)
+        return fail(IPT_ERR_INVALID, "ipt_scene_update_triangles: " + std::to_string(n_triangles) + " triangles given, the scene has " +
+                                         std::to_string(s->bvh.n) + " (a different count needs a new scene)");
+    CUDA_TRY(cudaSetDevice(s->device));
+    // a mislabelled pointer must be refused here: read from the other side it would fault
+    cudaPointerAttributes pa{};
+    if (cudaPointerGetAttributes(&pa, triangles) != cudaSuccess) {
+        cudaGetLastError();
+        pa.type = cudaMemoryTypeUnregistered;
+    }
+    const bool device_input = flags & IPT_UPDATE_DEVICE_POINTER;
+    if (device_input && !((pa.type == cudaMemoryTypeDevice || pa.type == cudaMemoryTypeManaged) && pa.device == s->device))
+        return fail(IPT_ERR_INVALID, "ipt_scene_update_triangles: IPT_UPDATE_DEVICE_POINTER given, but `triangles` is not device or managed "
+                                     "memory on the scene's device " + std::to_string(s->device));
+    if (!device_input && pa.type == cudaMemoryTypeDevice)
+        return fail(IPT_ERR_INVALID, "ipt_scene_update_triangles: `triangles` is device memory: pass IPT_UPDATE_DEVICE_POINTER");
+    if (reinterpret_cast<uintptr_t>(triangles) % alignof(float))
+        return fail(IPT_ERR_INVALID, "ipt_scene_update_triangles: `triangles` is not aligned to a float");
+    const uint32_t n = s->bvh.n;
+    DevBuf<float> staged;
+    const float* d_tris = triangles;
+    if (!device_input) { // the copy lbvh_build_host makes at scene creation
+        CUDA_TRY(staged.alloc(9 * (size_t)n));
+        CUDA_TRY(cudaMemcpyAsync(staged.p, triangles, sizeof(float) * 9 * (size_t)n, cudaMemcpyHostToDevice, s->stream));
+        d_tris = staged.p;
+    }
+    std::string err;
+    if (flags & IPT_UPDATE_REBUILD) {
+        // into a new tree: the scene keeps the old one unless the build succeeds. lbvh_build waits for the scene stream, so
+        // no enqueued render still reads the old buffers when they are freed.
+        LbvhDevice fresh;
+        if (lbvh_build(d_tris, n, s->stream, fresh, err) != 0) return fail(IPT_ERR_CUDA, "ipt_scene_update_triangles: LBVH build failed: " + err);
+        lbvh_free(s->bvh);
+        s->bvh = fresh;
+    } else if (lbvh_refit(d_tris, s->stream, s->bvh, err) != 0) {
+        return fail(IPT_ERR_CUDA, "ipt_scene_update_triangles: LBVH refit failed: " + err);
+    }
+    bind_mesh(s);
     return IPT_OK;
 }
 

@@ -303,20 +303,69 @@ __global__ void k_lbvh_compact(const BvhNode* __restrict__ nodes, uint32_t n_nod
     out[i] = q;
 }
 
+// leaf -> parent links of an existing tree, for a refit: each internal node writes the entry of its leaf children (the
+// parent links of internal nodes are kept in BvhNode::parent)
+__global__ void k_lbvh_leaf_parents(const BvhNode* __restrict__ nodes, uint32_t n_nodes, uint32_t* leaf_parent) {
+    uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_nodes) return;
+    uint32_t l = nodes[i].left, r = nodes[i].right;
+    if (l & 0x80000000u) leaf_parent[l & 0x7FFFFFFFu] = i;
+    if (r & 0x80000000u) leaf_parent[r & 0x7FFFFFFFu] = i;
+}
+
 static inline void lbvh_free(LbvhDevice& b) {
     cudaFree(b.tri_records); cudaFree(b.sorted_ids); cudaFree(b.sorted_keys); cudaFree(b.nodes); cudaFree(b.qnodes);
     b = LbvhDevice();
 }
 
-// Builds the LBVH for n triangles given in HOST memory (9 floats each). Returns 0 on success.
-static inline int lbvh_build(const float* host_tris, uint32_t n, cudaStream_t st, LbvhDevice& out, std::string& err, const float* host_extra = nullptr) {
 #define LB_TRY(expr)                                                     \
     do {                                                                 \
         cudaError_t e__ = (expr);                                        \
         if (e__ != cudaSuccess) { err = std::string(#expr) + ": " + cudaGetErrorString(e__); goto fail; } \
     } while (0)
-    float* d_tris = nullptr;
-    float* d_extra = nullptr;
+
+// Shared by build and refit, over the kept sorted order and topology: the internal boxes bottom-up from the leaf boxes
+// (lo, hi: tight boxes per original triangle; flags: n words of scratch) and the 64-byte records of the sorted triangles.
+static inline cudaError_t lbvh_fit(const float* tris, const float* extra, const float4* lo, const float4* hi, const uint32_t* leaf_parent,
+                                   uint32_t* flags, LbvhDevice& b, cudaStream_t st) {
+    const uint32_t n = b.n;
+    const unsigned blocks = (n + 255) / 256;
+    k_lbvh_records<<<blocks, 256, 0, st>>>(tris, b.sorted_ids, n, b.tri_records, extra);
+    if (n > 1) {
+        cudaError_t e = cudaMemsetAsync(flags, 0, 4 * (size_t)n, st);
+        if (e != cudaSuccess) return e;
+        k_lbvh_refit<<<blocks, 256, 0, st>>>(lo, hi, b.sorted_ids, n, b.nodes, leaf_parent, flags);
+    }
+    return cudaGetLastError();
+}
+
+// Shared by build and refit: the grid of the 32-byte nodes spans the root box (the union of the root's two child boxes);
+// quantises b.nodes into b.qnodes under it. Waits for the stream.
+static inline int lbvh_grid_compact(LbvhDevice& b, cudaStream_t st, std::string& err) {
+    if (b.n < 2) return 0;
+    BvhNode root;
+    LB_TRY(cudaMemcpyAsync(&root, b.nodes, sizeof root, cudaMemcpyDeviceToHost, st));
+    LB_TRY(cudaStreamSynchronize(st));
+    {
+        const float rlo[3] = {std::fmin(root.lo0x, root.lo1x), std::fmin(root.lo0y, root.lo1y), std::fmin(root.lo0z, root.lo1z)};
+        const float rhi[3] = {std::fmax(root.hi0x, root.hi1x), std::fmax(root.hi0y, root.hi1y), std::fmax(root.hi0z, root.hi1z)};
+        for (int a = 0; a < 3; ++a) {
+            float ext = rhi[a] - rlo[a];
+            b.grid.lo[a] = rlo[a];
+            b.grid.scale[a] = ext > 0.0f ? IPT_GRID_FILL / ext : 1.0f; // a flat scene: every coordinate maps to 1
+        }
+    }
+    k_lbvh_compact<<<(b.n - 1 + 255) / 256, 256, 0, st>>>(b.nodes, b.n - 1, b.grid, b.qnodes);
+    LB_TRY(cudaGetLastError());
+    LB_TRY(cudaStreamSynchronize(st));
+    return 0;
+fail:
+    return 1;
+}
+
+// Builds the LBVH for n triangles (9 floats each) and their optional per-primitive extras, both in DEVICE memory on the
+// stream's device. Returns 0 on success; on failure `out` holds nothing.
+static inline int lbvh_build(const float* d_tris, uint32_t n, cudaStream_t st, LbvhDevice& out, std::string& err, const float* d_extra = nullptr) {
     float4 *d_lo = nullptr, *d_hi = nullptr;
     uint32_t *d_cb = nullptr, *d_ids2 = nullptr, *d_counters = nullptr, *d_leaf_parent = nullptr, *d_flags = nullptr;
     unsigned long long* d_keys2 = nullptr;
@@ -325,12 +374,6 @@ static inline int lbvh_build(const float* host_tris, uint32_t n, cudaStream_t st
     out = LbvhDevice();
     out.n = n;
     {
-        LB_TRY(cudaMalloc((void**)&d_tris, sizeof(float) * 9 * (size_t)n));
-        LB_TRY(cudaMemcpyAsync(d_tris, host_tris, sizeof(float) * 9 * (size_t)n, cudaMemcpyHostToDevice, st));
-        if (host_extra) {
-            LB_TRY(cudaMalloc((void**)&d_extra, sizeof(float) * 3 * (size_t)n));
-            LB_TRY(cudaMemcpyAsync(d_extra, host_extra, sizeof(float) * 3 * (size_t)n, cudaMemcpyHostToDevice, st));
-        }
         LB_TRY(cudaMalloc((void**)&d_lo, 16 * (size_t)n));
         LB_TRY(cudaMalloc((void**)&d_hi, 16 * (size_t)n));
         LB_TRY(cudaMalloc((void**)&d_cb, 24));
@@ -355,41 +398,73 @@ static inline int lbvh_build(const float* host_tris, uint32_t n, cudaStream_t st
         }
         LB_TRY(cudaGetLastError());
         LB_TRY(cudaMalloc((void**)&out.tri_records, 64 * (size_t)n));
-        k_lbvh_records<<<blocks, 256, 0, st>>>(d_tris, out.sorted_ids, n, out.tri_records, d_extra);
         if (n > 1) {
             LB_TRY(cudaMalloc((void**)&out.nodes, sizeof(BvhNode) * (size_t)(n - 1)));
             LB_TRY(cudaMemsetAsync(out.nodes, 0, sizeof(BvhNode) * (size_t)(n - 1), st));
+            LB_TRY(cudaMalloc((void**)&out.qnodes, sizeof(BvhNodeQ) * (size_t)(n - 1)));
             LB_TRY(cudaMalloc((void**)&d_leaf_parent, 4 * (size_t)n));
             LB_TRY(cudaMalloc((void**)&d_flags, 4 * (size_t)n));
-            LB_TRY(cudaMemsetAsync(d_flags, 0, 4 * (size_t)n, st));
             k_lbvh_hierarchy<<<blocks, 256, 0, st>>>(out.sorted_keys, n, out.nodes, d_leaf_parent);
-            k_lbvh_refit<<<blocks, 256, 0, st>>>(d_lo, d_hi, out.sorted_ids, n, out.nodes, d_leaf_parent, d_flags);
-            // the grid of the 32-byte nodes spans the root box = the union of the root's two child boxes
-            BvhNode root;
-            LB_TRY(cudaMemcpyAsync(&root, out.nodes, sizeof root, cudaMemcpyDeviceToHost, st));
-            LB_TRY(cudaStreamSynchronize(st));
-            const float rlo[3] = {std::fmin(root.lo0x, root.lo1x), std::fmin(root.lo0y, root.lo1y), std::fmin(root.lo0z, root.lo1z)};
-            const float rhi[3] = {std::fmax(root.hi0x, root.hi1x), std::fmax(root.hi0y, root.hi1y), std::fmax(root.hi0z, root.hi1z)};
-            for (int a = 0; a < 3; ++a) {
-                float ext = rhi[a] - rlo[a];
-                out.grid.lo[a] = rlo[a];
-                out.grid.scale[a] = ext > 0.0f ? IPT_GRID_FILL / ext : 1.0f; // a flat scene: every coordinate maps to 1
-            }
-            LB_TRY(cudaMalloc((void**)&out.qnodes, sizeof(BvhNodeQ) * (size_t)(n - 1)));
-            k_lbvh_compact<<<(n - 1 + 255) / 256, 256, 0, st>>>(out.nodes, n - 1, out.grid, out.qnodes);
         }
-        LB_TRY(cudaGetLastError());
+        LB_TRY(lbvh_fit(d_tris, d_extra, d_lo, d_hi, d_leaf_parent, d_flags, out, st));
+        if (lbvh_grid_compact(out, st, err)) goto fail;
         LB_TRY(cudaStreamSynchronize(st));
     }
-    cudaFree(d_extra); cudaFree(d_tris); cudaFree(d_lo); cudaFree(d_hi); cudaFree(d_cb); cudaFree(d_keys2); cudaFree(d_ids2);
+    cudaFree(d_lo); cudaFree(d_hi); cudaFree(d_cb); cudaFree(d_keys2); cudaFree(d_ids2);
     cudaFree(d_counters); cudaFree(d_leaf_parent); cudaFree(d_flags);
     return 0;
 fail:
-    cudaFree(d_extra); cudaFree(d_tris); cudaFree(d_lo); cudaFree(d_hi); cudaFree(d_cb); cudaFree(d_keys2); cudaFree(d_ids2);
+    cudaFree(d_lo); cudaFree(d_hi); cudaFree(d_cb); cudaFree(d_keys2); cudaFree(d_ids2);
     cudaFree(d_counters); cudaFree(d_leaf_parent); cudaFree(d_flags);
     lbvh_free(out);
     return 1;
-#undef LB_TRY
 }
+
+// The same from HOST memory: the triangles (and extras) are staged on the stream, then built.
+static inline int lbvh_build_host(const float* host_tris, uint32_t n, cudaStream_t st, LbvhDevice& out, std::string& err,
+                                  const float* host_extra = nullptr) {
+    float* d_tris = nullptr;
+    float* d_extra = nullptr;
+    int rc = 1;
+    out = LbvhDevice();
+    LB_TRY(cudaMalloc((void**)&d_tris, sizeof(float) * 9 * (size_t)n));
+    LB_TRY(cudaMemcpyAsync(d_tris, host_tris, sizeof(float) * 9 * (size_t)n, cudaMemcpyHostToDevice, st));
+    if (host_extra) {
+        LB_TRY(cudaMalloc((void**)&d_extra, sizeof(float) * 3 * (size_t)n));
+        LB_TRY(cudaMemcpyAsync(d_extra, host_extra, sizeof(float) * 3 * (size_t)n, cudaMemcpyHostToDevice, st));
+    }
+    rc = lbvh_build(d_tris, n, st, out, err, d_extra);
+fail:
+    cudaFree(d_extra); cudaFree(d_tris);
+    return rc;
+}
+
+// Refit: new vertices (DEVICE memory, the triangle count of the tree) under the tree's kept topology and sorted order.
+// Recomputes the leaf boxes, the internal boxes, the records, the grid and the 32-byte nodes in place; the Morton keys and
+// sorted order stay those of the build. All scratch is allocated before anything of `b` is written: on an allocation
+// failure `b` is unchanged. Returns 0 on success.
+static inline int lbvh_refit(const float* d_tris, cudaStream_t st, LbvhDevice& b, std::string& err) {
+    const uint32_t n = b.n;
+    float4 *d_lo = nullptr, *d_hi = nullptr;
+    uint32_t *d_cb = nullptr, *d_leaf_parent = nullptr, *d_flags = nullptr;
+    int rc = 1;
+    LB_TRY(cudaMalloc((void**)&d_lo, 16 * (size_t)n));
+    LB_TRY(cudaMalloc((void**)&d_hi, 16 * (size_t)n));
+    LB_TRY(cudaMalloc((void**)&d_cb, 24)); // the centre bounds k_lbvh_bounds also gathers: unused here
+    if (n > 1) {
+        LB_TRY(cudaMalloc((void**)&d_leaf_parent, 4 * (size_t)n));
+        LB_TRY(cudaMalloc((void**)&d_flags, 4 * (size_t)n));
+        k_lbvh_leaf_parents<<<(n - 1 + 255) / 256, 256, 0, st>>>(b.nodes, n - 1, d_leaf_parent);
+    }
+    k_lbvh_bounds<<<(n + 255) / 256, 256, 0, st>>>(d_tris, n, d_lo, d_hi, d_cb, nullptr);
+    LB_TRY(lbvh_fit(d_tris, nullptr, d_lo, d_hi, d_leaf_parent, d_flags, b, st));
+    if (lbvh_grid_compact(b, st, err)) goto fail;
+    LB_TRY(cudaStreamSynchronize(st));
+    rc = 0;
+fail:
+    cudaFree(d_lo); cudaFree(d_hi); cudaFree(d_cb); cudaFree(d_leaf_parent); cudaFree(d_flags);
+    return rc;
+}
+#undef LB_TRY
 
 } // namespace iptd
