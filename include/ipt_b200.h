@@ -211,7 +211,7 @@ int ipt_scene_dispatch(ipt_scene* scene, uint32_t out[IPT_DISPATCH_WORDS]);
 
 /* Moving a mesh without recreating the scene (its stream, workspace and planes stay). */
 enum ipt_update_flags {
-    IPT_UPDATE_DEVICE_POINTER = 1u, /* `triangles` is device memory on the scene's device (e.g. a CUDA tensor) */
+    IPT_UPDATE_DEVICE_POINTER = 1u, /* the input is device memory on the scene's device (e.g. a CUDA tensor) */
     IPT_UPDATE_REBUILD = 2u         /* full LBVH build over the new vertices; default: refit the existing tree */
 };
 /* Replace the vertices of the scene's triangle mesh (9 floats per triangle, v0 e1 e2, as in ipt_scene_desc).
@@ -231,8 +231,29 @@ enum ipt_update_flags {
  *     scene's, and a pointer whose kind does not match the flag (by cudaPointerGetAttributes: with
  *     IPT_UPDATE_DEVICE_POINTER it must be device or managed memory on the scene's device, without it it must not be
  *     device memory), or that is not aligned to a float.
- *   Atomicity: if an allocation fails (IPT_ERR_CUDA), the scene keeps its previous triangles and tree. */
+ *   Atomicity: if an allocation fails (IPT_ERR_CUDA), the scene keeps its previous triangles and tree.
+ *   Per-triangle materials set by ipt_scene_set_triangle_materials stay with their triangles, after a refit and a rebuild. */
 int ipt_scene_update_triangles(ipt_scene* scene, const float* triangles, uint64_t n_triangles, uint32_t flags);
+
+/* Give each triangle of the scene's mesh its own material. materials[k] indexes the material list the scene was created
+ * with, for triangle k in the order of ipt_scene_desc::triangles (the triangle whose primitive id is n_prims + k).
+ * n_triangles must equal the scene's count.
+ *   Flags: only IPT_UPDATE_DEVICE_POINTER: `materials` is then device or managed memory on the scene's device (e.g. a CUDA
+ *     tensor of int32 or uint32).
+ *   Result: afterwards every render and ipt_mix_sample equals what a scene whose triangle k has material materials[k] would
+ *     give. ipt_trace_batch, ipt_preview_batch, ipt_bvh_export* and ipt_scene_dispatch do not change. Until the first call,
+ *     every triangle has ipt_scene_desc::triangle_material.
+ *   Persistence: a material belongs to its original triangle index and is kept through ipt_scene_update_triangles, refit
+ *     and rebuild alike. A later call replaces the whole array.
+ *   Synchronisation: as ipt_scene_update_triangles: takes the scene's mutex, runs on the scene's stream after the work
+ *     already enqueued there and returns once the call is complete. With IPT_UPDATE_DEVICE_POINTER the caller must have
+ *     finished writing the buffer on its own stream before the call.
+ *   Planes made on the scene stay valid, and their accumulators are not touched.
+ *   Errors (IPT_ERR_INVALID): a null argument, unknown flag bits, a scene without a mesh, a count that differs from the
+ *     scene's, a pointer whose kind does not match the flag (as for ipt_scene_update_triangles) or that is not 4-byte
+ *     aligned, and any index >= the scene's n_materials (device input is checked on the device before anything changes).
+ *   Atomicity: on any error, including a failed allocation (IPT_ERR_CUDA), the scene keeps the materials it had. */
+int ipt_scene_set_triangle_materials(ipt_scene* scene, const uint32_t* materials, uint64_t n_triangles, uint32_t flags);
 
 /* The reference's five scenes + this repo's benchmark scenes as descriptions:
  * "box" (make_scene_box, the default), "fractal", "smallpt", "square", "corner", "openspheres", "cornell" (C2),

@@ -102,6 +102,7 @@ SIGNATURES = {
     "ipt_scene_set_camera": (C.c_int, [_vp, C.POINTER(Camera)]),
     "ipt_scene_dispatch": (C.c_int, [_vp, u32p]),
     "ipt_scene_update_triangles": (C.c_int, [_vp, _vp, C.c_uint64, C.c_uint32]),
+    "ipt_scene_set_triangle_materials": (C.c_int, [_vp, _vp, C.c_uint64, C.c_uint32]),
     "ipt_sample_scene": (C.c_int, [C.c_char_p, C.POINTER(C.POINTER(SceneDesc))]),
     "ipt_scene_desc_free": (C.c_int, [C.POINTER(SceneDesc)]),
     "ipt_light_derived": (C.c_int, [C.POINTER(Light), f32p, f32p, f32p]),
@@ -318,6 +319,32 @@ class Scene:
             raise ValueError(f"triangles: shape (n, 9) or (9n,) required, got {shape}")
         n = shape[0] if len(shape) == 2 else shape[0] // 9
         check(load().ipt_scene_update_triangles(self.handle, ptr, n, flags))
+
+    def set_triangle_materials(self, materials):
+        """ipt_scene_set_triangle_materials: materials[k] (an index into the scene's material list) for triangle k of the
+        mesh. `materials` is a C-contiguous uint32 numpy array of length n (host input), or a contiguous int32 or uint32
+        CUDA tensor of length n on the scene's device (device input: torch's current stream on that device is synchronised
+        first). Kept through update_triangles; a later call replaces the whole array."""
+        flags = 0
+        if isinstance(materials, np.ndarray):
+            if materials.dtype != np.uint32 or not materials.flags.c_contiguous:
+                raise TypeError("materials: a C-contiguous uint32 array is required")
+            shape, ptr = materials.shape, materials.ctypes.data
+        else:
+            import torch  # device input, as in update_triangles
+
+            if not isinstance(materials, torch.Tensor):
+                raise TypeError(f"materials: a numpy array or a CUDA tensor is required, not {type(materials).__name__}")
+            if materials.dtype not in (torch.int32, torch.uint32) or not materials.is_contiguous():
+                raise TypeError("materials: a contiguous int32 or uint32 tensor is required")
+            if materials.device.type != "cuda" or materials.device.index != self.device:
+                raise ValueError(f"materials: a tensor on cuda:{self.device} (the scene's device) is required, not on {materials.device}")
+            torch.cuda.current_stream(materials.device).synchronize()
+            shape, ptr = tuple(materials.shape), materials.data_ptr()
+            flags |= UPDATE_DEVICE_POINTER
+        if len(shape) != 1:
+            raise ValueError(f"materials: shape (n,) required, got {shape}")
+        check(load().ipt_scene_set_triangle_materials(self.handle, ptr, shape[0], flags))
 
     def trace_batch(self, origins, directions):
         o, d = _f32(origins).reshape(-1, 3), _f32(directions).reshape(-1, 3)

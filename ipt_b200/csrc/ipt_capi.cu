@@ -116,6 +116,10 @@ struct ipt_scene {
     float* d_light_samp = nullptr;
     DevMaterial* d_mats = nullptr;
     LbvhDevice bvh{};
+    // per-triangle materials, null until ipt_scene_set_triangle_materials: the caller's array (by original triangle index)
+    // and its gather into the tree's sorted order (DevScene::tri_mats), redone by every rebuild
+    uint32_t* d_tri_mats_orig = nullptr;
+    uint32_t* d_tri_mats = nullptr;
     LbvhDevice light_bvh{};
     bool smallpt = false, mesh = false;
     SceneSpec shade_spec = SPEC_RUNTIME; // k_shade<FUSE_NEXT / FUSE_LAST, ., shade_spec>
@@ -257,6 +261,14 @@ __global__ void k_philox_batch(const uint4* __restrict__ c, size_t n, PhiloxKeys
     uint4 r = philox4x32(c[i].x, c[i].y, c[i].z, c[i].w, keys);
     if (blocks) blocks[i] = r;
     if (uniforms) uniforms[i] = make_float4(u01(r.x), u01(r.y), u01(r.z), u01(r.w));
+}
+
+// *out = max(*out, max of v[0..n)): the range check of device-resident material indices
+__global__ void k_max_u32(const uint32_t* __restrict__ v, size_t n, uint32_t* out) {
+    uint32_t m = 0;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) m = max(m, v[i]);
+    for (int off = 16; off > 0; off >>= 1) m = max(m, __shfl_xor_sync(0xffffffffu, m, off));
+    if ((threadIdx.x & 31) == 0) atomicMax(out, m);
 }
 
 __global__ void k_plane_add_rays(RenderCtx C, size_t n, const float* __restrict__ x, const float* __restrict__ y, const float* __restrict__ v) {
@@ -440,6 +452,25 @@ static void bind_mesh(ipt_scene* s) {
     s->dev.nodes = s->bvh.nodes;
     s->dev.qnodes = s->bvh.qnodes;
     s->dev.grid = s->bvh.grid;
+    s->dev.tri_mats = s->d_tri_mats;
+}
+
+// The input pointer of an entry that takes host or device memory (IPT_UPDATE_DEVICE_POINTER). A mislabelled pointer must be
+// refused here: read from the other side it would fault. `align_what` names the required alignment in the message.
+static int check_input_pointer(const ipt_scene* s, const void* p, bool device_input, size_t align, const char* entry, const char* arg,
+                               const char* align_what) {
+    cudaPointerAttributes pa{};
+    if (cudaPointerGetAttributes(&pa, p) != cudaSuccess) {
+        cudaGetLastError();
+        pa.type = cudaMemoryTypeUnregistered;
+    }
+    const std::string who = std::string(entry) + ": `" + arg + "`";
+    if (device_input && !((pa.type == cudaMemoryTypeDevice || pa.type == cudaMemoryTypeManaged) && pa.device == s->device))
+        return fail(IPT_ERR_INVALID, std::string(entry) + ": IPT_UPDATE_DEVICE_POINTER given, but `" + arg +
+                                         "` is not device or managed memory on the scene's device " + std::to_string(s->device));
+    if (!device_input && pa.type == cudaMemoryTypeDevice) return fail(IPT_ERR_INVALID, who + " is device memory: pass IPT_UPDATE_DEVICE_POINTER");
+    if (reinterpret_cast<uintptr_t>(p) % align) return fail(IPT_ERR_INVALID, who + " is not aligned to " + align_what);
+    return IPT_OK;
 }
 
 static size_t stack_smem(const ipt_scene* s) { return s->mesh ? (size_t)IPT_STACK_SHORT * IPT_BLOCK * sizeof(uint32_t) : 0; }
@@ -714,6 +745,7 @@ int ipt_scene_destroy(ipt_scene* s) {
     free_workspace(s->ws);
     lbvh_free(s->bvh);
     lbvh_free(s->light_bvh);
+    cudaFree(s->d_tri_mats_orig); cudaFree(s->d_tri_mats);
     cudaFree(s->d_prims); cudaFree(s->d_lights); cudaFree(s->d_light_cdf); cudaFree(s->d_light_guide); cudaFree(s->d_light_samp); cudaFree(s->d_mats); cudaFree(s->d_cnt); cudaFree(s->d_stats);
     if (s->pinned) cudaFreeHost(s->pinned);
     for (cudaEvent_t e : s->events) cudaEventDestroy(e);
@@ -755,20 +787,8 @@ int ipt_scene_update_triangles(ipt_scene* s, const float* triangles, uint64_t n_
         return fail(IPT_ERR_INVALID, "ipt_scene_update_triangles: " + std::to_string(n_triangles) + " triangles given, the scene has " +
                                          std::to_string(s->bvh.n) + " (a different count needs a new scene)");
     CUDA_TRY(cudaSetDevice(s->device));
-    // a mislabelled pointer must be refused here: read from the other side it would fault
-    cudaPointerAttributes pa{};
-    if (cudaPointerGetAttributes(&pa, triangles) != cudaSuccess) {
-        cudaGetLastError();
-        pa.type = cudaMemoryTypeUnregistered;
-    }
     const bool device_input = flags & IPT_UPDATE_DEVICE_POINTER;
-    if (device_input && !((pa.type == cudaMemoryTypeDevice || pa.type == cudaMemoryTypeManaged) && pa.device == s->device))
-        return fail(IPT_ERR_INVALID, "ipt_scene_update_triangles: IPT_UPDATE_DEVICE_POINTER given, but `triangles` is not device or managed "
-                                     "memory on the scene's device " + std::to_string(s->device));
-    if (!device_input && pa.type == cudaMemoryTypeDevice)
-        return fail(IPT_ERR_INVALID, "ipt_scene_update_triangles: `triangles` is device memory: pass IPT_UPDATE_DEVICE_POINTER");
-    if (reinterpret_cast<uintptr_t>(triangles) % alignof(float))
-        return fail(IPT_ERR_INVALID, "ipt_scene_update_triangles: `triangles` is not aligned to a float");
+    if (int rc = check_input_pointer(s, triangles, device_input, alignof(float), "ipt_scene_update_triangles", "triangles", "a float")) return rc;
     const uint32_t n = s->bvh.n;
     DevBuf<float> staged;
     const float* d_tris = triangles;
@@ -780,14 +800,74 @@ int ipt_scene_update_triangles(ipt_scene* s, const float* triangles, uint64_t n_
     std::string err;
     if (flags & IPT_UPDATE_REBUILD) {
         // into a new tree: the scene keeps the old one unless the build succeeds. lbvh_build waits for the scene stream, so
-        // no enqueued render still reads the old buffers when they are freed.
+        // no enqueued render still reads the old buffers when they are freed. Per-triangle materials follow the new sorted
+        // order: their buffer is allocated before the build and filled from it before the swap.
+        DevBuf<uint32_t> mats;
+        if (s->d_tri_mats_orig) CUDA_TRY(mats.alloc(n));
         LbvhDevice fresh;
         if (lbvh_build(d_tris, n, s->stream, fresh, err) != 0) return fail(IPT_ERR_CUDA, "ipt_scene_update_triangles: LBVH build failed: " + err);
+        if (mats.p) {
+            k_lbvh_gather<<<(n + 255) / 256, 256, 0, s->stream>>>(s->d_tri_mats_orig, fresh.sorted_ids, n, mats.p);
+            cudaError_t e = cudaGetLastError();
+            if (e == cudaSuccess) e = cudaStreamSynchronize(s->stream);
+            if (e != cudaSuccess) {
+                lbvh_free(fresh);
+                return fail(IPT_ERR_CUDA, std::string("ipt_scene_update_triangles: material gather failed: ") + cudaGetErrorString(e));
+            }
+            cudaFree(s->d_tri_mats);
+            s->d_tri_mats = mats.p;
+            mats.p = nullptr;
+        }
         lbvh_free(s->bvh);
         s->bvh = fresh;
     } else if (lbvh_refit(d_tris, s->stream, s->bvh, err) != 0) {
         return fail(IPT_ERR_CUDA, "ipt_scene_update_triangles: LBVH refit failed: " + err);
     }
+    bind_mesh(s);
+    return IPT_OK;
+}
+
+int ipt_scene_set_triangle_materials(ipt_scene* s, const uint32_t* materials, uint64_t n_triangles, uint32_t flags) {
+    static const char* entry = "ipt_scene_set_triangle_materials";
+    if (!s || !materials) return fail(IPT_ERR_INVALID, std::string(entry) + ": null argument");
+    if (flags & ~(uint32_t)IPT_UPDATE_DEVICE_POINTER) return fail(IPT_ERR_INVALID, std::string(entry) + ": unknown flag bits " + std::to_string(flags));
+    std::lock_guard<std::recursive_mutex> lock__(s->mu);
+    if (!s->mesh) return fail(IPT_ERR_INVALID, std::string(entry) + ": the scene has no triangle mesh");
+    if (n_triangles != s->bvh.n)
+        return fail(IPT_ERR_INVALID, std::string(entry) + ": " + std::to_string(n_triangles) + " materials given, the scene has " +
+                                         std::to_string(s->bvh.n) + " triangles");
+    CUDA_TRY(cudaSetDevice(s->device));
+    const bool device_input = flags & IPT_UPDATE_DEVICE_POINTER;
+    if (int rc = check_input_pointer(s, materials, device_input, alignof(uint32_t), entry, "materials", "4 bytes")) return rc;
+    const uint32_t n = s->bvh.n, n_mats = s->dev.n_materials;
+    if (!device_input)
+        for (uint32_t k = 0; k < n; ++k)
+            if (materials[k] >= n_mats)
+                return fail(IPT_ERR_INVALID, std::string(entry) + ": materials[" + std::to_string(k) + "] = " + std::to_string(materials[k]) +
+                                                 " is out of range: the scene has " + std::to_string(n_mats) + " materials");
+    // new buffers, filled and checked before anything of the scene changes
+    DevBuf<uint32_t> orig, sorted, max_word;
+    CUDA_TRY(orig.alloc(n));
+    CUDA_TRY(sorted.alloc(n));
+    if (device_input) CUDA_TRY(max_word.alloc(1));
+    CUDA_TRY(cudaMemcpyAsync(orig.p, materials, sizeof(uint32_t) * (size_t)n, device_input ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, s->stream));
+    if (device_input) {
+        uint32_t max_index = 0;
+        CUDA_TRY(cudaMemsetAsync(max_word.p, 0, sizeof(uint32_t), s->stream));
+        k_max_u32<<<std::min<uint32_t>((n + 255) / 256, 4 * (uint32_t)s->sm_count), 256, 0, s->stream>>>(orig.p, n, max_word.p);
+        CUDA_TRY(cudaGetLastError());
+        CUDA_TRY(cudaMemcpyAsync(&max_index, max_word.p, sizeof(uint32_t), cudaMemcpyDeviceToHost, s->stream));
+        CUDA_TRY(cudaStreamSynchronize(s->stream));
+        if (max_index >= n_mats)
+            return fail(IPT_ERR_INVALID, std::string(entry) + ": a material index is out of range (largest " + std::to_string(max_index) +
+                                             "): the scene has " + std::to_string(n_mats) + " materials");
+    }
+    k_lbvh_gather<<<(n + 255) / 256, 256, 0, s->stream>>>(orig.p, s->bvh.sorted_ids, n, sorted.p);
+    CUDA_TRY(cudaGetLastError());
+    // the stream is idle after this: no enqueued render still reads the buffers replaced below
+    CUDA_TRY(cudaStreamSynchronize(s->stream));
+    std::swap(s->d_tri_mats_orig, orig.p);
+    std::swap(s->d_tri_mats, sorted.p);
     bind_mesh(s);
     return IPT_OK;
 }

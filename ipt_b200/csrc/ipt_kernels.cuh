@@ -498,14 +498,17 @@ __global__ void __launch_bounds__(256, IPT_EXTEND_MIN_BLOCKS) k_extend(const __g
     flush_stat(C.stats, ST_LIGHT_NODES, tc.light_nodes);
 }
 
-// geometric normal + material of a hit primitive (GeometrySphereInBox.cpp:43-56 and the other geometries)
+// geometric normal + material of a hit primitive (GeometrySphereInBox.cpp:43-56 and the other geometries).
+// TRI_MATS = false for kernels that never shade a mesh hit (the fused shade kernels: mesh scenes run the unfused loop).
+template <bool TRI_MATS = true>
 __device__ __forceinline__ void surface_frame(const DevScene& S, uint32_t prim, f3 pos, f3& normal, uint32_t& material) {
     if (prim >= S.n_prims) {
         uint32_t k = prim - S.n_prims; // sorted triangle position
         float4 a = __ldg(&S.tris[4 * (size_t)k]);
         float4 b = __ldg(&S.tris[4 * (size_t)k + 1]);
         normal = mk3(a.w, b.x, b.y);
-        material = S.tri_material;
+        // a uniform branch: the pointer is a kernel parameter
+        material = TRI_MATS && S.tri_mats ? __ldg(S.tri_mats + k) : S.tri_material;
         return;
     }
     // the index differs per lane: a constant-bank read would serialise, a global (L1-cached) read does not
@@ -686,7 +689,7 @@ __global__ void __launch_bounds__(256, FUSE == FUSE_LAST ? IPT_SHADE_FUSED_MIN_B
             pixel = iy * C.width + ix;
             f3 normal;
             uint32_t material;
-            surface_frame(S, b.y, pos, normal, material);
+            surface_frame<FUSE == FUSE_NONE>(S, b.y, pos, normal, material);
             const float4* mp = reinterpret_cast<const float4*>(&S.mats_g[material]);
             float4 m0 = __ldg(mp), m1 = __ldg(mp + 1);
             DevMaterial m;

@@ -313,6 +313,12 @@ __global__ void k_lbvh_leaf_parents(const BvhNode* __restrict__ nodes, uint32_t 
     if (r & 0x80000000u) leaf_parent[r & 0x7FFFFFFFu] = i;
 }
 
+// a per-triangle value (by original index) into the tree's sorted order: sorted[k] = orig[sorted_ids[k]]
+__global__ void k_lbvh_gather(const uint32_t* __restrict__ orig, const uint32_t* __restrict__ sorted_ids, uint32_t n, uint32_t* sorted) {
+    uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k < n) sorted[k] = orig[sorted_ids[k]];
+}
+
 static inline void lbvh_free(LbvhDevice& b) {
     cudaFree(b.tri_records); cudaFree(b.sorted_ids); cudaFree(b.sorted_keys); cudaFree(b.nodes); cudaFree(b.qnodes);
     b = LbvhDevice();
