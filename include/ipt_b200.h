@@ -209,10 +209,10 @@ int ipt_scene_set_camera(ipt_scene* scene, const ipt_camera* camera);
 #define IPT_DISPATCH_WORDS 7
 int ipt_scene_dispatch(ipt_scene* scene, uint32_t out[IPT_DISPATCH_WORDS]);
 
-/* Moving a mesh without recreating the scene (its stream, workspace and planes stay). */
+/* Moving a mesh or the lights without recreating the scene (its stream, workspace and planes stay). */
 enum ipt_update_flags {
     IPT_UPDATE_DEVICE_POINTER = 1u, /* the input is device memory on the scene's device (e.g. a CUDA tensor) */
-    IPT_UPDATE_REBUILD = 2u         /* full LBVH build over the new vertices; default: refit the existing tree */
+    IPT_UPDATE_REBUILD = 2u         /* full LBVH build over the new vertices or lights; default: refit the existing tree */
 };
 /* Replace the vertices of the scene's triangle mesh (9 floats per triangle, v0 e1 e2, as in ipt_scene_desc).
  * n_triangles must equal the scene's count; a different count needs a new scene. Lights are not moved.
@@ -254,6 +254,33 @@ int ipt_scene_update_triangles(ipt_scene* scene, const float* triangles, uint64_
  *     aligned, and any index >= the scene's n_materials (device input is checked on the device before anything changes).
  *   Atomicity: on any error, including a failed allocation (IPT_ERR_CUDA), the scene keeps the materials it had. */
 int ipt_scene_set_triangle_materials(ipt_scene* scene, const uint32_t* materials, uint64_t n_triangles, uint32_t flags);
+
+/* Move and re-power the scene's lights without recreating the scene: each light's position, axes, radius and power may
+ * change. n_lights must equal the scene's count, and lights[i].kind the kind of the scene's light i: count and kinds decide
+ * the kernels ipt_scene_create chose, so a change of either needs a new scene.
+ *   Flags: IPT_UPDATE_DEVICE_POINTER: `lights` is device or managed memory on the scene's device (e.g. a CUDA tensor of
+ *     48-byte ipt_light records). IPT_UPDATE_REBUILD: build the light LBVH anew; by default the existing tree is refitted.
+ *     A scene without a light LBVH accepts IPT_UPDATE_REBUILD and has nothing to rebuild.
+ *   Result: afterwards every result (traces, ipt_light_ddf_*, ipt_mix_sample, renders, ipt_scene_dispatch) equals that of
+ *     a scene created from the same description with the new lights; after a rebuild bit for bit. A refit keeps the light
+ *     tree's topology and sorted order and only recomputes every box and record, so two things may differ from a fresh
+ *     scene: the light tree's traversal counters of renders (light_bvh_nodes_visited, and lights_tested, which counts the
+ *     tree's leaves reached), and the order in which the all-hits mixture density is summed over the lights a
+ *     direction crosses, so the density (ipt_light_ddf_value, the mixture value of ipt_mix_sample, the child weights of a
+ *     render) may differ in the last bits where a direction crosses more than one light. The nearest light is exact (ties
+ *     go to the lower original index). Of ipt_scene_dispatch only out[4] (lights_inside_box) can change.
+ *   Synchronisation: as ipt_scene_update_triangles: takes the scene's mutex, runs on the scene's stream after the work
+ *     already enqueued there and returns once the update is complete. With IPT_UPDATE_DEVICE_POINTER the caller must have
+ *     finished writing the buffer on its own stream before the call.
+ *   Planes made on the scene stay valid, and their accumulators are not touched. The mesh and per-triangle materials are
+ *     not touched.
+ *   Errors (IPT_ERR_INVALID): a null argument, unknown flag bits, a count that differs from the scene's, a kind that
+ *     differs from the scene's (the message names the first such index; device input is checked on the device before
+ *     anything changes), and a pointer whose kind does not match the flag (as for ipt_scene_update_triangles) or that is
+ *     not 4-byte aligned. Values are not range-checked, as ipt_scene_create does not check them.
+ *   Atomicity: on any error, including a failed allocation (IPT_ERR_CUDA), the scene keeps the lights, tables and light
+ *     tree it had. */
+int ipt_scene_update_lights(ipt_scene* scene, const ipt_light* lights, uint32_t n_lights, uint32_t flags);
 
 /* The reference's five scenes + this repo's benchmark scenes as descriptions:
  * "box" (make_scene_box, the default), "fractal", "smallpt", "square", "corner", "openspheres", "cornell" (C2),

@@ -103,6 +103,7 @@ SIGNATURES = {
     "ipt_scene_dispatch": (C.c_int, [_vp, u32p]),
     "ipt_scene_update_triangles": (C.c_int, [_vp, _vp, C.c_uint64, C.c_uint32]),
     "ipt_scene_set_triangle_materials": (C.c_int, [_vp, _vp, C.c_uint64, C.c_uint32]),
+    "ipt_scene_update_lights": (C.c_int, [_vp, _vp, C.c_uint32, C.c_uint32]),
     "ipt_sample_scene": (C.c_int, [C.c_char_p, C.POINTER(C.POINTER(SceneDesc))]),
     "ipt_scene_desc_free": (C.c_int, [C.POINTER(SceneDesc)]),
     "ipt_light_derived": (C.c_int, [C.POINTER(Light), f32p, f32p, f32p]),
@@ -345,6 +346,33 @@ class Scene:
         if len(shape) != 1:
             raise ValueError(f"materials: shape (n,) required, got {shape}")
         check(load().ipt_scene_set_triangle_materials(self.handle, ptr, shape[0], flags))
+
+    def update_lights(self, lights, rebuild: bool = False):
+        """ipt_scene_update_lights: new positions, axes, radii and powers for the scene's lights, same count and kinds.
+        `lights` is a sequence of Light (host input), or a contiguous float32 or int32 CUDA tensor of shape (n, 12) on the
+        scene's device laid out as ipt_light records, column 0 holding the kind's bit pattern (device input: torch's current
+        stream on that device is synchronised first). rebuild=False refits the light LBVH, rebuild=True builds it anew."""
+        flags = UPDATE_REBUILD if rebuild else 0
+        if isinstance(lights, (list, tuple)):
+            if not all(isinstance(l, Light) for l in lights):
+                raise TypeError("lights: a sequence of capi.Light is required")
+            arr = (Light * len(lights))(*lights)
+            n, ptr = len(lights), C.addressof(arr)
+        else:
+            import torch  # device input, as in update_triangles
+
+            if not isinstance(lights, torch.Tensor):
+                raise TypeError(f"lights: a sequence of capi.Light or a CUDA tensor is required, not {type(lights).__name__}")
+            if lights.dtype not in (torch.float32, torch.int32) or not lights.is_contiguous():
+                raise TypeError("lights: a contiguous float32 or int32 tensor is required")
+            if lights.device.type != "cuda" or lights.device.index != self.device:
+                raise ValueError(f"lights: a tensor on cuda:{self.device} (the scene's device) is required, not on {lights.device}")
+            if lights.dim() != 2 or lights.shape[1] != C.sizeof(Light) // 4:
+                raise ValueError(f"lights: shape (n, {C.sizeof(Light) // 4}) required, got {tuple(lights.shape)}")
+            torch.cuda.current_stream(lights.device).synchronize()
+            n, ptr = lights.shape[0], lights.data_ptr()
+            flags |= UPDATE_DEVICE_POINTER
+        check(load().ipt_scene_update_lights(self.handle, ptr, n, flags))
 
     def trace_batch(self, origins, directions):
         o, d = _f32(origins).reshape(-1, 3), _f32(directions).reshape(-1, 3)

@@ -271,6 +271,142 @@ __global__ void k_max_u32(const uint32_t* __restrict__ v, size_t n, uint32_t* ou
     if ((threadIdx.x & 31) == 0) atomicMax(out, m);
 }
 
+// ---------------------------------------------------------------------------------------------------
+// light derivation on the device (ipt_scene_update_lights): the bytes flatten_lights and ipt_scene_create upload, in
+// their operation order (the host side is compiled with -ffp-contract=off; here every step is an explicit _rn intrinsic)
+// ---------------------------------------------------------------------------------------------------
+// One thread per light: the DevLight record (weight and cdf follow in k_light_weights / k_light_scan), the 64-byte record
+// of DevScene::light_samp and, for a scene with a light LBVH, the tree's inputs: 9 floats and (kind, area, weight). The
+// area-light arithmetic is that of k_lbvh_records (AreaLight::AreaLight, lighting.cpp:79-90). A kind that differs from
+// the scene's light i is reported by the smallest such index in *mismatch.
+__global__ void k_light_derive(const ipt_light* __restrict__ in, uint32_t n, const DevLight* __restrict__ current, DevLight* out, float4* samp,
+                               float* ltris, float* extra, uint32_t* mismatch) {
+    uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const ipt_light l = in[i];
+    if (l.kind != current[i].kind) atomicMin(mismatch, i);
+    DevLight o{};
+    o.kind = l.kind;
+    o.power = l.power;
+    o.px = l.position[0]; o.py = l.position[1]; o.pz = l.position[2];
+    o.radius = l.radius;
+    o.xax = l.x_axis[0]; o.xay = l.x_axis[1]; o.xaz = l.x_axis[2];
+    o.yax = l.y_axis[0]; o.yay = l.y_axis[1]; o.yaz = l.y_axis[2];
+    if (l.kind == IPT_LIGHT_AREA_DIAMOND || l.kind == IPT_LIGHT_AREA_TRIANGLE) {
+        const f3 e1 = mk3(o.xax, o.xay, o.xaz), e2 = mk3(o.yax, o.yay, o.yaz);
+        const f3 cr = xcross3(e1, e2);
+        const float full_area = xlength3(cr);
+        o.area = l.kind == IPT_LIGHT_AREA_DIAMOND ? full_area : xdiv(full_area, 2.0f);
+        // glm::inverse(mat3(e1, e2, cr)) rows 0 and 1, as k_lbvh_records
+        float m00 = e1.x, m01 = e1.y, m02 = e1.z, m10 = e2.x, m11 = e2.y, m12 = e2.z, m20 = cr.x, m21 = cr.y, m22 = cr.z;
+        float det = xadd(xsub(xmul(m00, xsub(xmul(m11, m22), xmul(m21, m12))), xmul(m10, xsub(xmul(m01, m22), xmul(m21, m02)))),
+                         xmul(m20, xsub(xmul(m01, m12), xmul(m11, m02))));
+        float ood = xdiv(1.0f, det);
+        o.i0x = xmul(xsub(xmul(m11, m22), xmul(m21, m12)), ood);
+        o.i0y = xmul(-xsub(xmul(m10, m22), xmul(m20, m12)), ood);
+        o.i0z = xmul(xsub(xmul(m10, m21), xmul(m20, m11)), ood);
+        o.i1x = xmul(-xsub(xmul(m01, m22), xmul(m21, m02)), ood);
+        o.i1y = xmul(xsub(xmul(m00, m22), xmul(m20, m02)), ood);
+        o.i1z = xmul(-xsub(xmul(m00, m21), xmul(m20, m01)), ood);
+        const f3 nn = xnormalize3(cr);
+        o.nx = nn.x; o.ny = nn.y; o.nz = nn.z;
+        o.surface_power = xdiv(l.power, o.area);
+    } else if (l.kind == IPT_LIGHT_SPHERE || l.kind == IPT_LIGHT_SPHERE_INVERTED) {
+        const double r = (double)l.radius; // lighting.h:51, in double as the host evaluates 4.0 * M_PI * r * r
+        o.area = __double2float_rn(__dmul_rn(__dmul_rn(4.0 * M_PI, r), r));
+        o.surface_power = xdiv(l.power, o.area);
+    } else if (l.kind == IPT_LIGHT_POINT) {
+        o.area = 0.0f;
+        o.surface_power = __uint_as_float(0x7FC00000u); // the host's NAN (lighting.cpp:204)
+    }
+    out[i] = o;
+    samp[4 * (size_t)i] = make_float4(o.px, o.py, o.pz, __uint_as_float(o.kind));
+    samp[4 * (size_t)i + 1] = make_float4(o.xax, o.xay, o.xaz, o.radius);
+    samp[4 * (size_t)i + 2] = make_float4(o.yax, o.yay, o.yaz, 0.0f);
+    samp[4 * (size_t)i + 3] = make_float4(o.nx, o.ny, o.nz, 0.0f);
+    if (ltris) {
+        float* t = ltris + 9 * (size_t)i;
+        t[0] = o.px; t[1] = o.py; t[2] = o.pz;
+        t[3] = o.xax; t[4] = o.xay; t[5] = o.xaz;
+        t[6] = o.yax; t[7] = o.yay; t[8] = o.yaz;
+        extra[3 * (size_t)i] = l.kind == IPT_LIGHT_AREA_TRIANGLE ? 1.0f : 0.0f;
+        extra[3 * (size_t)i + 1] = o.area;
+    }
+}
+
+// The mixture weights of flatten_lights' unite() loop: appending light j rescales every earlier weight by
+// f_j = ka_j / (ka_j + p_j) and gives light j the weight r_j = p_j / (ka_j + p_j), where ka_j is the running float sum of
+// the powers before j. So w_i = r_i * f_{i+1} * ... * f_{n-1} * 0.5, multiplied left to right. Three stages keep every
+// rounding: ka in order (one thread), f and r (one thread each), and each weight's chain of multiplies in order.
+__global__ void k_light_power_prefix(const ipt_light* __restrict__ in, uint32_t n, float* ka) {
+    if (blockIdx.x || threadIdx.x) return;
+    float acc = 0.0f;
+    for (uint32_t j = 0; j < n; ++j) {
+        ka[j] = acc;
+        acc = xadd(acc, in[j].power);
+    }
+}
+
+__global__ void k_light_ratios(const ipt_light* __restrict__ in, const float* __restrict__ ka, uint32_t n, float* f, float* r) {
+    uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n) return;
+    const float a = ka[j], p = in[j].power, s = xadd(a, p);
+    f[j] = xdiv(a, s);
+    r[j] = xdiv(p, s);
+}
+
+// Four consecutive lights per thread: each f_j is loaded once for the four chains, which are independent multiplies.
+// No reassociation: light i still multiplies r_i by f_{i+1}, f_{i+2}, ... in that order, then by 0.5 (main.cpp:143).
+#define IPT_WEIGHTS_PER_THREAD 4
+__global__ void k_light_weights(const float* __restrict__ f, const float* __restrict__ r, uint32_t n, float* w, DevLight* out, float* extra) {
+    const uint32_t i0 = IPT_WEIGHTS_PER_THREAD * (blockIdx.x * blockDim.x + threadIdx.x);
+    if (i0 >= n) return;
+    float c[IPT_WEIGHTS_PER_THREAD];
+#pragma unroll
+    for (int k = 0; k < IPT_WEIGHTS_PER_THREAD; ++k) c[k] = i0 + k < n ? r[i0 + k] : 0.0f;
+    const uint32_t common = min(i0 + IPT_WEIGHTS_PER_THREAD, n);
+    for (uint32_t j = i0 + 1; j < common; ++j) {
+        const float fj = f[j];
+#pragma unroll
+        for (int k = 0; k < IPT_WEIGHTS_PER_THREAD; ++k)
+            if (i0 + k < j) c[k] = xmul(c[k], fj);
+    }
+#pragma unroll 4
+    for (uint32_t j = common; j < n; ++j) {
+        const float fj = f[j];
+#pragma unroll
+        for (int k = 0; k < IPT_WEIGHTS_PER_THREAD; ++k) c[k] = xmul(c[k], fj);
+    }
+#pragma unroll
+    for (int k = 0; k < IPT_WEIGHTS_PER_THREAD; ++k) {
+        const uint32_t i = i0 + k;
+        if (i >= n) break;
+        const float wi = xmul(c[k], 0.5f);
+        w[i] = wi;
+        out[i].weight = wi;
+        if (extra) extra[3 * (size_t)i + 2] = wi;
+    }
+}
+
+// The running float sum of the weights (DevLight::cdf, DevScene::light_cdf) and the guide table, in one thread: the sum
+// keeps its order, and guide[b] is the host's monotone search, whose result on plateaus of the cdf (zero powers) is the
+// contract.
+__global__ void k_light_scan(const float* __restrict__ w, uint32_t n, float* cdf, DevLight* out, uint32_t* guide) {
+    if (blockIdx.x || threadIdx.x) return;
+    float acc = 0.0f;
+    for (uint32_t i = 0; i < n; ++i) {
+        acc = xadd(acc, w[i]);
+        cdf[i] = acc;
+        out[i].cdf = acc;
+    }
+    uint32_t i = 0;
+    for (uint32_t b = 0; b <= IPT_LIGHT_GUIDE + 1; ++b) {
+        const float edge = xdiv((float)b, (float)IPT_LIGHT_GUIDE);
+        while (i < n && !(edge < cdf[i])) ++i;
+        guide[b] = i;
+    }
+}
+
 __global__ void k_plane_add_rays(RenderCtx C, size_t n, const float* __restrict__ x, const float* __restrict__ y, const float* __restrict__ v) {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
@@ -473,6 +609,32 @@ static int check_input_pointer(const ipt_scene* s, const void* p, bool device_in
     return IPT_OK;
 }
 
+// grouped box planes + inline spheres only (analytic_closest's first branch)
+static bool geom_fast_scene(const ipt_scene* s) { return !s->smallpt && !s->mesh && s->dev.planes_grouped && s->dev.others_inline; }
+
+// DevScene::lights_inside_box. Shadow rays of box scenes skip the wall planes: every non-plane primitive is a sphere inside
+// the closed box [-1,1]^3 and every light is an area light whose corners keep a margin of 1e-3 to every wall, so origin (a
+// point of a wall or of a sphere) and target lie in the convex box and no wall can come between them. `box_area_light`: a
+// geom_fast scene whose lights are the inline ones, all of them area lights.
+static uint32_t lights_inside_box(const DevScene& dv, bool box_area_light, const ipt_light* lights, uint32_t n_lights) {
+    if (!box_area_light || dv.n_planes == 0) return 0;
+    bool inside = true;
+    for (uint32_t k = 0; k < dv.n_others; ++k) {
+        const DevSphere& sp = dv.others[k];
+        const float r = std::sqrt(sp.r2);
+        for (float c : {sp.cx, sp.cy, sp.cz}) inside = inside && std::fabs(c) + r <= 1.0f;
+    }
+    for (uint32_t i = 0; i < n_lights; ++i) {
+        const ipt_light& l = lights[i];
+        for (int corner = 0; corner < 4; ++corner)
+            for (int a = 0; a < 3; ++a) {
+                const float q = l.position[a] + ((corner & 1) ? l.x_axis[a] : 0.0f) + ((corner & 2) ? l.y_axis[a] : 0.0f);
+                inside = inside && std::fabs(q) <= 1.0f - 1e-3f;
+            }
+    }
+    return inside ? 1u : 0u;
+}
+
 static size_t stack_smem(const ipt_scene* s) { return s->mesh ? (size_t)IPT_STACK_SHORT * IPT_BLOCK * sizeof(uint32_t) : 0; }
 
 template <class T>
@@ -635,28 +797,8 @@ int ipt_scene_create(const ipt_scene_desc* desc, int device, ipt_scene** out) {
     s->smallpt = smallpt;
     s->mesh = desc->n_triangles > 0;
     // grouped box planes + inline spheres only (analytic_closest's first branch)
-    const bool geom_fast = !smallpt && !s->mesh && dv.planes_grouped && dv.others_inline;
-    // Shadow rays of box scenes skip the wall planes (DevScene::lights_inside_box): every non-plane primitive is a sphere
-    // inside the closed box [-1,1]^3 and every light is an area light whose corners keep a margin of 1e-3 to every wall, so
-    // origin (a point of a wall or of a sphere) and target lie in the convex box and no wall can come between them.
-    dv.lights_inside_box = 0;
-    if (geom_fast && inline_area_light && dv.n_planes > 0) {
-        bool inside = true;
-        for (uint32_t k = 0; k < dv.n_others; ++k) {
-            const DevSphere& sp = dv.others[k];
-            const float r = std::sqrt(sp.r2);
-            for (float c : {sp.cx, sp.cy, sp.cz}) inside = inside && std::fabs(c) + r <= 1.0f;
-        }
-        for (uint32_t i = 0; i < desc->n_lights; ++i) {
-            const ipt_light& l = desc->lights[i];
-            for (int corner = 0; corner < 4; ++corner)
-                for (int a = 0; a < 3; ++a) {
-                    const float q = l.position[a] + ((corner & 1) ? l.x_axis[a] : 0.0f) + ((corner & 2) ? l.y_axis[a] : 0.0f);
-                    inside = inside && std::fabs(q) <= 1.0f - 1e-3f;
-                }
-        }
-        dv.lights_inside_box = inside ? 1u : 0u;
-    }
+    const bool geom_fast = geom_fast_scene(s);
+    dv.lights_inside_box = lights_inside_box(dv, geom_fast && inline_area_light, desc->lights, desc->n_lights);
     bool all_lambert = true; // every material is the cosine DDF
     for (const DevMaterial& m : mats) if (m.ddf != IPT_DDF_COSINE) all_lambert = false;
     if (s->mesh) {
@@ -869,6 +1011,110 @@ int ipt_scene_set_triangle_materials(ipt_scene* s, const uint32_t* materials, ui
     std::swap(s->d_tri_mats_orig, orig.p);
     std::swap(s->d_tri_mats, sorted.p);
     bind_mesh(s);
+    return IPT_OK;
+}
+
+int ipt_scene_update_lights(ipt_scene* s, const ipt_light* lights, uint32_t n_lights, uint32_t flags) {
+    static const char* entry = "ipt_scene_update_lights";
+    if (!s || !lights) return fail(IPT_ERR_INVALID, std::string(entry) + ": null argument");
+    if (flags & ~(uint32_t)(IPT_UPDATE_DEVICE_POINTER | IPT_UPDATE_REBUILD))
+        return fail(IPT_ERR_INVALID, std::string(entry) + ": unknown flag bits " + std::to_string(flags));
+    std::lock_guard<std::recursive_mutex> lock__(s->mu);
+    DevScene& dv = s->dev;
+    if (n_lights != dv.n_lights)
+        return fail(IPT_ERR_INVALID, std::string(entry) + ": " + std::to_string(n_lights) + " lights given, the scene has " +
+                                         std::to_string(dv.n_lights) + " (a different count needs a new scene)");
+    CUDA_TRY(cudaSetDevice(s->device));
+    const bool device_input = flags & IPT_UPDATE_DEVICE_POINTER;
+    if (int rc = check_input_pointer(s, lights, device_input, alignof(uint32_t), entry, "lights", "4 bytes")) return rc;
+    const uint32_t n = n_lights;
+    if (n == 0) return IPT_OK;
+    const bool tree = dv.n_light_bvh > 0;
+    // new buffers, filled and checked before anything of the scene changes
+    DevBuf<ipt_light> staged;
+    DevBuf<DevLight> d_lights;
+    DevBuf<float> cdf, samp, scratch, ltris, extra;
+    DevBuf<uint32_t> guide, word;
+    CUDA_TRY(d_lights.alloc(n));
+    CUDA_TRY(cdf.alloc(n));
+    CUDA_TRY(samp.alloc(16 * (size_t)n));
+    CUDA_TRY(scratch.alloc(4 * (size_t)n)); // ka, f, r, w
+    CUDA_TRY(guide.alloc(IPT_LIGHT_GUIDE + 2));
+    CUDA_TRY(word.alloc(1));
+    if (tree) {
+        CUDA_TRY(ltris.alloc(9 * (size_t)n));
+        CUDA_TRY(extra.alloc(3 * (size_t)n));
+    }
+    const ipt_light* d_in = lights;
+    if (!device_input) {
+        CUDA_TRY(staged.alloc(n));
+        CUDA_TRY(cudaMemcpyAsync(staged.p, lights, sizeof(ipt_light) * (size_t)n, cudaMemcpyHostToDevice, s->stream));
+        d_in = staged.p;
+    }
+    float *ka = scratch.p, *f = ka + n, *r = f + n, *w = r + n;
+    const unsigned blocks = (n + 255) / 256;
+    CUDA_TRY(cudaMemsetAsync(word.p, 0xFF, sizeof(uint32_t), s->stream));
+    k_light_derive<<<blocks, 256, 0, s->stream>>>(d_in, n, s->d_lights, d_lights.p, reinterpret_cast<float4*>(samp.p), ltris.p, extra.p, word.p);
+    k_light_power_prefix<<<1, 1, 0, s->stream>>>(d_in, n, ka);
+    k_light_ratios<<<blocks, 256, 0, s->stream>>>(d_in, ka, n, f, r);
+    const uint32_t weight_threads = (n + IPT_WEIGHTS_PER_THREAD - 1) / IPT_WEIGHTS_PER_THREAD;
+    k_light_weights<<<(weight_threads + 127) / 128, 128, 0, s->stream>>>(f, r, n, w, d_lights.p, extra.p);
+    k_light_scan<<<1, 1, 0, s->stream>>>(w, n, cdf.p, d_lights.p, guide.p);
+    CUDA_TRY(cudaGetLastError());
+    // what the host needs back: the kind check and, for a scene that holds its light inline, the derived record and the
+    // input record (DevScene::lights and lights_inside_box)
+    uint32_t first_bad = 0;
+    DevLight inline_derived[IPT_INLINE_LIGHTS];
+    ipt_light inline_input[IPT_INLINE_LIGHTS];
+    const uint32_t n_inline = dv.light_inline ? n : 0; // n <= IPT_INLINE_LIGHTS
+    CUDA_TRY(cudaMemcpyAsync(&first_bad, word.p, sizeof first_bad, cudaMemcpyDeviceToHost, s->stream));
+    if (n_inline) {
+        CUDA_TRY(cudaMemcpyAsync(inline_derived, d_lights.p, sizeof(DevLight) * n_inline, cudaMemcpyDeviceToHost, s->stream));
+        CUDA_TRY(cudaMemcpyAsync(inline_input, d_in, sizeof(ipt_light) * n_inline, cudaMemcpyDeviceToHost, s->stream));
+    }
+    CUDA_TRY(cudaStreamSynchronize(s->stream));
+    if (first_bad != 0xFFFFFFFFu)
+        return fail(IPT_ERR_INVALID, std::string(entry) + ": lights[" + std::to_string(first_bad) + "].kind differs from the kind of the scene's light " +
+                                         std::to_string(first_bad) + " (a different kind needs a new scene)");
+    // the light LBVH: a rebuild goes into a new tree, swapped in only if the build succeeds; a refit allocates all its scratch
+    // before it writes the tree
+    LbvhDevice fresh;
+    bool rebuilt = false;
+    if (tree) {
+        std::string err;
+        if (flags & IPT_UPDATE_REBUILD) {
+            if (lbvh_build(ltris.p, n, s->stream, fresh, err, extra.p) != 0) return fail(IPT_ERR_CUDA, std::string(entry) + ": light LBVH build failed: " + err);
+            rebuilt = true;
+        } else if (lbvh_refit(ltris.p, s->stream, s->light_bvh, err, extra.p) != 0) {
+            return fail(IPT_ERR_CUDA, std::string(entry) + ": light LBVH refit failed: " + err);
+        }
+    }
+    // commit. The stream is idle (the tree stages end with a synchronise): no enqueued render still reads the buffers that
+    // are replaced, and the DevBufs free them on return.
+    std::swap(s->d_lights, d_lights.p);
+    std::swap(s->d_light_cdf, cdf.p);
+    std::swap(s->d_light_guide, guide.p);
+    std::swap(s->d_light_samp, samp.p);
+    dv.lights_g = s->d_lights;
+    dv.light_cdf = s->d_light_cdf;
+    dv.light_guide = s->d_light_guide;
+    dv.light_samp = reinterpret_cast<const float4*>(s->d_light_samp);
+    if (rebuilt) {
+        lbvh_free(s->light_bvh);
+        s->light_bvh = fresh;
+    }
+    if (tree) {
+        dv.light_nodes = s->light_bvh.nodes;
+        dv.light_qnodes = s->light_bvh.qnodes;
+        dv.light_grid = s->light_bvh.grid;
+        dv.light_recs = s->light_bvh.tri_records;
+    }
+    bool inline_area_light = n_inline > 0;
+    for (uint32_t i = 0; i < n_inline; ++i) {
+        dv.lights[i] = inline_derived[i];
+        if (inline_input[i].kind > IPT_LIGHT_AREA_TRIANGLE) inline_area_light = false;
+    }
+    dv.lights_inside_box = lights_inside_box(dv, geom_fast_scene(s) && inline_area_light, inline_input, n_inline);
     return IPT_OK;
 }
 

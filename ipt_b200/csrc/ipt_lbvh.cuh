@@ -448,8 +448,9 @@ fail:
 // Refit: new vertices (DEVICE memory, the triangle count of the tree) under the tree's kept topology and sorted order.
 // Recomputes the leaf boxes, the internal boxes, the records, the grid and the 32-byte nodes in place; the Morton keys and
 // sorted order stay those of the build. All scratch is allocated before anything of `b` is written: on an allocation
-// failure `b` is unchanged. Returns 0 on success.
-static inline int lbvh_refit(const float* d_tris, cudaStream_t st, LbvhDevice& b, std::string& err) {
+// failure `b` is unchanged. Returns 0 on success. A light tree passes its per-primitive extras (DEVICE memory, as for
+// lbvh_build): the boxes of diamonds then take the fourth corner, and the records carry kind, area and weight.
+static inline int lbvh_refit(const float* d_tris, cudaStream_t st, LbvhDevice& b, std::string& err, const float* d_extra = nullptr) {
     const uint32_t n = b.n;
     float4 *d_lo = nullptr, *d_hi = nullptr;
     uint32_t *d_cb = nullptr, *d_leaf_parent = nullptr, *d_flags = nullptr;
@@ -462,8 +463,8 @@ static inline int lbvh_refit(const float* d_tris, cudaStream_t st, LbvhDevice& b
         LB_TRY(cudaMalloc((void**)&d_flags, 4 * (size_t)n));
         k_lbvh_leaf_parents<<<(n - 1 + 255) / 256, 256, 0, st>>>(b.nodes, n - 1, d_leaf_parent);
     }
-    k_lbvh_bounds<<<(n + 255) / 256, 256, 0, st>>>(d_tris, n, d_lo, d_hi, d_cb, nullptr);
-    LB_TRY(lbvh_fit(d_tris, nullptr, d_lo, d_hi, d_leaf_parent, d_flags, b, st));
+    k_lbvh_bounds<<<(n + 255) / 256, 256, 0, st>>>(d_tris, n, d_lo, d_hi, d_cb, d_extra);
+    LB_TRY(lbvh_fit(d_tris, d_extra, d_lo, d_hi, d_leaf_parent, d_flags, b, st));
     if (lbvh_grid_compact(b, st, err)) goto fail;
     LB_TRY(cudaStreamSynchronize(st));
     rc = 0;
