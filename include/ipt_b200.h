@@ -353,6 +353,15 @@ int ipt_bvh_export(ipt_scene* scene, ipt_bvh_node* nodes, uint32_t* sorted_prims
  * coordinate (x - lo) * scale * 65536 + 4. Integer work + three float steps: byte-identical to the CPU restatement. */
 int ipt_bvh_export_compact(ipt_scene* scene, uint32_t* nodes32, float grid[6], uint64_t* n_nodes);
 
+/* The scene's light tables as the render kernels read them, for the scene's n_lights lights in description order: Light::area,
+ * power / area (NaN for point lights), the normal of an area light (3 floats per light, zero for the other kinds), the
+ * weight of the light in the mixture of main.cpp:142-143 (CollectionLighting.cpp:12-21 weights, halved) and the running
+ * float sum of those weights (cdf); and the light-selection guide: guide[b] = the first i with b / 4096 < cdf[i]
+ * (n_lights if none), b = 0 .. IPT_LIGHT_GUIDE_WORDS - 1. HOST arrays; any output may be NULL. */
+#define IPT_LIGHT_GUIDE_WORDS 4098
+int ipt_light_tables_export(ipt_scene* scene, float* area, float* surface_power, float* normal, float* weight, float* cdf,
+                            uint32_t guide[IPT_LIGHT_GUIDE_WORDS]);
+
 /* ---- render plane: replaces RenderPlane::addRay accumulation (tracer_interfaces.h:51-54) --------- */
 int ipt_plane_create(ipt_scene* scene, uint32_t width, uint32_t height, ipt_plane** out);
 /* Accumulate into caller-owned DEVICE arrays (e.g. torch tensors that NCCL will all-reduce). */

@@ -22,6 +22,7 @@ SPEC_FEW_LIGHTS, SPEC_LIGHT_BVH, SPEC_RUNTIME, SPEC_ONE_LIGHT, SPEC_ONE_AREA_LIG
 DISPATCH_FIELDS = ("spec", "smallpt", "mesh", "mesh_box_scene", "lights_inside_box", "light_inline", "n_light_bvh")
 DISPATCH_WORDS = len(DISPATCH_FIELDS)
 UPDATE_DEVICE_POINTER, UPDATE_REBUILD = 1, 2  # ipt_update_flags
+LIGHT_GUIDE_WORDS = 4098  # IPT_LIGHT_GUIDE_WORDS: entries of the light-selection guide
 
 import os
 
@@ -119,6 +120,7 @@ SIGNATURES = {
     "ipt_philox_batch": (C.c_int, [C.c_int, u32p, C.c_size_t, C.c_uint64, u32p, f32p]),
     "ipt_bvh_export": (C.c_int, [_vp, C.POINTER(BvhNode), u32p, u64p, u64p]),
     "ipt_bvh_export_compact": (C.c_int, [_vp, u32p, f32p, u64p]),
+    "ipt_light_tables_export": (C.c_int, [_vp, f32p, f32p, f32p, f32p, f32p, u32p]),
     "ipt_plane_create": (C.c_int, [_vp, C.c_uint32, C.c_uint32, C.POINTER(_vp)]),
     "ipt_plane_wrap": (C.c_int, [_vp, C.c_uint32, C.c_uint32, _vp, _vp, _vp, C.POINTER(_vp)]),
     "ipt_plane_clear": (C.c_int, [_vp]),
@@ -443,6 +445,16 @@ class Scene:
         nodes = np.zeros((n.value, 8), np.uint32); grid = np.zeros(6, np.float32)
         check(load().ipt_bvh_export_compact(self.handle, _ptr(nodes, u32p), _ptr(grid, f32p), C.byref(n)))
         return nodes, grid
+
+    def light_tables(self):
+        """The light tables the kernels read: dict of area, surface_power, normal (n, 3), weight, cdf (float32) and the
+        light-selection guide (uint32[LIGHT_GUIDE_WORDS])."""
+        n = self.description.desc.n_lights
+        t = dict(area=np.empty(n, np.float32), surface_power=np.empty(n, np.float32), normal=np.empty((n, 3), np.float32),
+                 weight=np.empty(n, np.float32), cdf=np.empty(n, np.float32), guide=np.empty(LIGHT_GUIDE_WORDS, np.uint32))
+        check(load().ipt_light_tables_export(self.handle, *(_ptr(t[k], f32p) for k in ("area", "surface_power", "normal", "weight", "cdf")),
+                                             _ptr(t["guide"], u32p)))
+        return t
 
     def render_host(self, params: RenderParams, out=None):
         """The end-to-end call: host buffers in, host buffers out. `out` = (sum, sumsq, count) arrays to reuse."""

@@ -1,8 +1,9 @@
 // ipt_capi.cu — the C ABI of include/ipt_b200.h: scene flattening, workspace management, the per-batch
 // kernel sequence of the wavefront pipeline, and the parity entry points.
 //
-// Host-side float work (light areas/normals/inverse matrices, mixture weights) follows the reference's
-// constructors in glm operation order (ipt_b200/host/glm_order.hpp) so the device consumes the same bits.
+// The scene's light tables are derived on the device (k_light_derive and the kernels after it), for ipt_scene_create
+// and ipt_scene_update_lights alike. Host-side float work (ipt_light_derived) follows the reference's constructors in glm
+// operation order (ipt_b200/host/glm_order.hpp) so it gives the same bits.
 #include "ipt_b200.h"
 
 #include "../host/glm_order.hpp"
@@ -272,19 +273,19 @@ __global__ void k_max_u32(const uint32_t* __restrict__ v, size_t n, uint32_t* ou
 }
 
 // ---------------------------------------------------------------------------------------------------
-// light derivation on the device (ipt_scene_update_lights): the bytes flatten_lights and ipt_scene_create upload, in
-// their operation order (the host side is compiled with -ffp-contract=off; here every step is an explicit _rn intrinsic)
+// the scene's light tables (derive_lights, for ipt_scene_create and ipt_scene_update_lights) in the reference's operation
+// order: every step is an explicit _rn intrinsic; oracle/ipt_oracle.c restates them (prepare_light, prepare_weights)
 // ---------------------------------------------------------------------------------------------------
 // One thread per light: the DevLight record (weight and cdf follow in k_light_weights / k_light_scan), the 64-byte record
 // of DevScene::light_samp and, for a scene with a light LBVH, the tree's inputs: 9 floats and (kind, area, weight). The
 // area-light arithmetic is that of k_lbvh_records (AreaLight::AreaLight, lighting.cpp:79-90). A kind that differs from
-// the scene's light i is reported by the smallest such index in *mismatch.
+// the scene's light i is reported by the smallest such index in *mismatch; a new scene has no lights yet (`current` null).
 __global__ void k_light_derive(const ipt_light* __restrict__ in, uint32_t n, const DevLight* __restrict__ current, DevLight* out, float4* samp,
                                float* ltris, float* extra, uint32_t* mismatch) {
     uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     const ipt_light l = in[i];
-    if (l.kind != current[i].kind) atomicMin(mismatch, i);
+    if (current && l.kind != current[i].kind) atomicMin(mismatch, i);
     DevLight o{};
     o.kind = l.kind;
     o.power = l.power;
@@ -334,10 +335,12 @@ __global__ void k_light_derive(const ipt_light* __restrict__ in, uint32_t n, con
     }
 }
 
-// The mixture weights of flatten_lights' unite() loop: appending light j rescales every earlier weight by
+// The mixture weights of CollectionLighting::distributionInPoint (src/CollectionLighting.cpp:12-21) through unite()'s
+// union+simple branch (src/libddf/ddf.cpp:207-223): appending light j rescales every earlier weight by
 // f_j = ka_j / (ka_j + p_j) and gives light j the weight r_j = p_j / (ka_j + p_j), where ka_j is the running float sum of
-// the powers before j. So w_i = r_i * f_{i+1} * ... * f_{n-1} * 0.5, multiplied left to right. Three stages keep every
-// rounding: ka in order (one thread), f and r (one thread each), and each weight's chain of multiplies in order.
+// the powers before j; main.cpp:143 then halves every weight. So w_i = r_i * f_{i+1} * ... * f_{n-1} * 0.5, multiplied
+// left to right. Three stages keep every rounding: ka in order (one thread), f and r (one thread each), and each weight's
+// chain of multiplies in order.
 __global__ void k_light_power_prefix(const ipt_light* __restrict__ in, uint32_t n, float* ka) {
     if (blockIdx.x || threadIdx.x) return;
     float acc = 0.0f;
@@ -389,8 +392,8 @@ __global__ void k_light_weights(const float* __restrict__ f, const float* __rest
 }
 
 // The running float sum of the weights (DevLight::cdf, DevScene::light_cdf) and the guide table, in one thread: the sum
-// keeps its order, and guide[b] is the host's monotone search, whose result on plateaus of the cdf (zero powers) is the
-// contract.
+// keeps its order, and guide[b] is a monotone search, whose result on plateaus of the cdf (zero powers) is the contract.
+// Without lights the guide is all zero.
 __global__ void k_light_scan(const float* __restrict__ w, uint32_t n, float* cdf, DevLight* out, uint32_t* guide) {
     if (blockIdx.x || threadIdx.x) return;
     float acc = 0.0f;
@@ -434,68 +437,6 @@ __global__ void k_plane_resolve(const float* __restrict__ sum, const uint32_t* _
 // ---------------------------------------------------------------------------------------------------
 // scene flattening
 // ---------------------------------------------------------------------------------------------------
-static int flatten_lights(const ipt_scene_desc* d, std::vector<DevLight>& out, float& sdf_weight) {
-    namespace H = ipt_host;
-    uint32_t n = d->n_lights;
-    out.assign(n, DevLight{});
-    std::vector<float> w(n);
-    // CollectionLighting::distributionInPoint (src/CollectionLighting.cpp:12-21) through unite()'s union+simple
-    // branch (src/libddf/ddf.cpp:207-223): every earlier weight is rescaled each time a light is appended.
-    float acc_power = 0.0f;
-    for (uint32_t j = 0; j < n; ++j) {
-        float ka = acc_power, kb = d->lights[j].power;
-        float f = ka / (ka + kb);
-        for (uint32_t i = 0; i < j; ++i) w[i] *= f;
-        w[j] = kb / (ka + kb);
-        acc_power += kb;
-    }
-    // main.cpp:143 unite(light_ddf, 1, sdf, 1); with no lights unite() degenerates to the sdf alone (ddf.cpp:209-210)
-    if (n == 0) sdf_weight = 1.0f;
-    else {
-        float f = 1.0f / (1.0f + 1.0f);
-        for (uint32_t i = 0; i < n; ++i) w[i] *= f;
-        sdf_weight = 1.0f / (1.0f + 1.0f);
-    }
-    float acc = 0.0f;
-    for (uint32_t i = 0; i < n; ++i) {
-        const ipt_light& l = d->lights[i];
-        DevLight& o = out[i];
-        o.kind = l.kind;
-        o.power = l.power;
-        o.px = l.position[0]; o.py = l.position[1]; o.pz = l.position[2];
-        o.radius = l.radius;
-        o.xax = l.x_axis[0]; o.xay = l.x_axis[1]; o.xaz = l.x_axis[2];
-        o.yax = l.y_axis[0]; o.yay = l.y_axis[1]; o.yaz = l.y_axis[2];
-        if (l.kind == IPT_LIGHT_AREA_DIAMOND || l.kind == IPT_LIGHT_AREA_TRIANGLE) {
-            // AreaLight::AreaLight (src/lighting/lighting.cpp:79-90)
-            H::f3 xa = H::mk(l.x_axis), ya = H::mk(l.y_axis);
-            H::f3 cr = H::cross(xa, ya);
-            float full_area = H::length(cr);
-            o.area = l.kind == IPT_LIGHT_AREA_DIAMOND ? full_area : full_area / 2.0f;
-            H::f33 m;
-            m.c[0] = xa; m.c[1] = ya; m.c[2] = cr;
-            H::f33 inv = H::inverse(m);
-            o.i0x = inv.c[0].x; o.i0y = inv.c[1].x; o.i0z = inv.c[2].x;
-            o.i1x = inv.c[0].y; o.i1y = inv.c[1].y; o.i1z = inv.c[2].y;
-            H::f3 nn = H::normalize(cr);
-            o.nx = nn.x; o.ny = nn.y; o.nz = nn.z;
-            o.surface_power = l.power / o.area;
-        } else if (l.kind == IPT_LIGHT_SPHERE || l.kind == IPT_LIGHT_SPHERE_INVERTED) {
-            o.area = (float)(4.0 * M_PI * l.radius * l.radius); // lighting.h:51
-            o.surface_power = l.power / o.area;
-        } else if (l.kind == IPT_LIGHT_POINT) {
-            o.area = 0.0f;
-            o.surface_power = NAN; // lighting.cpp:204
-        } else {
-            return fail(IPT_ERR_INVALID, "unknown light kind");
-        }
-        o.weight = w[i];
-        acc += w[i];
-        o.cdf = acc;
-    }
-    return IPT_OK;
-}
-
 static int flatten_prims(const ipt_scene_desc* d, std::vector<DevPrim>& out, bool& smallpt) {
     out.assign(d->n_prims, DevPrim{});
     smallpt = false;
@@ -644,6 +585,107 @@ struct DevBuf {
     cudaError_t alloc(size_t n) { return cudaMalloc((void**)&p, std::max<size_t>(n, 1) * sizeof(T)); }
 };
 
+// n elements of an entry's input on the device: `*d_p` is device memory as given, or host memory copied into `staged` on
+// the scene stream
+template <class T>
+static cudaError_t stage_input(const ipt_scene* s, const T* p, size_t n, bool device_input, DevBuf<T>& staged, const T** d_p) {
+    *d_p = p;
+    if (device_input) return cudaSuccess;
+    cudaError_t e = staged.alloc(n);
+    if (e == cudaSuccess && n) e = cudaMemcpyAsync(staged.p, p, sizeof(T) * n, cudaMemcpyHostToDevice, s->stream);
+    *d_p = staged.p;
+    return e;
+}
+
+// The scene's light tables from n ipt_light records in device memory, for ipt_scene_create and ipt_scene_update_lights:
+// the DevLight records, DevScene::light_cdf, light_guide and light_samp, the light LBVH of a scene that has one (built into
+// a new tree when `rebuild`, else refitted), the inline records and lights_inside_box. The scene's shape (n_lights,
+// light_inline, n_light_bvh) is decided already. Everything is derived into new buffers and checked before anything of the
+// scene changes; the kinds are checked against the scene's current lights, which a new scene does not have yet (its
+// d_lights is null). `who` starts the error messages.
+static int derive_lights(ipt_scene* s, const ipt_light* d_in, uint32_t n, bool rebuild, const std::string& who) {
+    DevScene& dv = s->dev;
+    const bool tree = dv.n_light_bvh > 0;
+    DevBuf<DevLight> d_lights;
+    DevBuf<float> cdf, samp, scratch, ltris, extra;
+    DevBuf<uint32_t> guide, word;
+    CUDA_TRY(d_lights.alloc(n));
+    CUDA_TRY(cdf.alloc(n));
+    CUDA_TRY(samp.alloc(16 * (size_t)n));
+    CUDA_TRY(scratch.alloc(4 * (size_t)n)); // ka, f, r, w
+    CUDA_TRY(guide.alloc(IPT_LIGHT_GUIDE + 2));
+    CUDA_TRY(word.alloc(1));
+    if (tree) {
+        CUDA_TRY(ltris.alloc(9 * (size_t)n));
+        CUDA_TRY(extra.alloc(3 * (size_t)n));
+    }
+    float *ka = scratch.p, *f = ka + n, *r = f + n, *w = r + n;
+    CUDA_TRY(cudaMemsetAsync(word.p, 0xFF, sizeof(uint32_t), s->stream));
+    if (n) { // a grid of zero blocks is a launch error: without lights only k_light_scan runs
+        const unsigned blocks = (n + 255) / 256;
+        k_light_derive<<<blocks, 256, 0, s->stream>>>(d_in, n, s->d_lights, d_lights.p, reinterpret_cast<float4*>(samp.p), ltris.p, extra.p, word.p);
+        k_light_power_prefix<<<1, 1, 0, s->stream>>>(d_in, n, ka);
+        k_light_ratios<<<blocks, 256, 0, s->stream>>>(d_in, ka, n, f, r);
+        const uint32_t weight_threads = (n + IPT_WEIGHTS_PER_THREAD - 1) / IPT_WEIGHTS_PER_THREAD;
+        k_light_weights<<<(weight_threads + 127) / 128, 128, 0, s->stream>>>(f, r, n, w, d_lights.p, extra.p);
+    }
+    k_light_scan<<<1, 1, 0, s->stream>>>(w, n, cdf.p, d_lights.p, guide.p);
+    CUDA_TRY(cudaGetLastError());
+    // what the host needs back: the kind check and, for a scene that holds its light inline, the derived record and the
+    // input record (DevScene::lights and lights_inside_box)
+    uint32_t first_bad = 0;
+    DevLight inline_derived[IPT_INLINE_LIGHTS];
+    ipt_light inline_input[IPT_INLINE_LIGHTS];
+    const uint32_t n_inline = dv.light_inline ? n : 0; // n <= IPT_INLINE_LIGHTS
+    CUDA_TRY(cudaMemcpyAsync(&first_bad, word.p, sizeof first_bad, cudaMemcpyDeviceToHost, s->stream));
+    if (n_inline) {
+        CUDA_TRY(cudaMemcpyAsync(inline_derived, d_lights.p, sizeof(DevLight) * n_inline, cudaMemcpyDeviceToHost, s->stream));
+        CUDA_TRY(cudaMemcpyAsync(inline_input, d_in, sizeof(ipt_light) * n_inline, cudaMemcpyDeviceToHost, s->stream));
+    }
+    CUDA_TRY(cudaStreamSynchronize(s->stream));
+    if (first_bad != 0xFFFFFFFFu)
+        return fail(IPT_ERR_INVALID, who + "lights[" + std::to_string(first_bad) + "].kind differs from the kind of the scene's light " +
+                                         std::to_string(first_bad) + " (a different kind needs a new scene)");
+    // the light LBVH: a rebuild goes into a new tree, swapped in only if the build succeeds; a refit allocates all its scratch
+    // before it writes the tree
+    LbvhDevice fresh;
+    if (tree) {
+        std::string err;
+        if (rebuild) {
+            if (lbvh_build(ltris.p, n, s->stream, fresh, err, extra.p) != 0) return fail(IPT_ERR_CUDA, who + "light LBVH build failed: " + err);
+        } else if (lbvh_refit(ltris.p, s->stream, s->light_bvh, err, extra.p) != 0) {
+            return fail(IPT_ERR_CUDA, who + "light LBVH refit failed: " + err);
+        }
+    }
+    // commit. The stream is idle (the read-back and the tree stages end with a synchronise): no enqueued render still reads
+    // the buffers that are replaced, and the DevBufs free them on return.
+    std::swap(s->d_lights, d_lights.p);
+    std::swap(s->d_light_cdf, cdf.p);
+    std::swap(s->d_light_guide, guide.p);
+    std::swap(s->d_light_samp, samp.p);
+    dv.lights_g = s->d_lights;
+    dv.light_cdf = s->d_light_cdf;
+    dv.light_guide = s->d_light_guide;
+    dv.light_samp = reinterpret_cast<const float4*>(s->d_light_samp);
+    if (tree && rebuild) {
+        lbvh_free(s->light_bvh);
+        s->light_bvh = fresh;
+    }
+    if (tree) {
+        dv.light_nodes = s->light_bvh.nodes;
+        dv.light_qnodes = s->light_bvh.qnodes;
+        dv.light_grid = s->light_bvh.grid;
+        dv.light_recs = s->light_bvh.tri_records;
+    }
+    bool inline_area_light = n_inline > 0;
+    for (uint32_t i = 0; i < n_inline; ++i) {
+        dv.lights[i] = inline_derived[i];
+        if (inline_input[i].kind > IPT_LIGHT_AREA_TRIANGLE) inline_area_light = false;
+    }
+    dv.lights_inside_box = lights_inside_box(dv, geom_fast_scene(s) && inline_area_light, inline_input, n_inline);
+    return IPT_OK;
+}
+
 extern "C" {
 
 int ipt_abi_version(void) { return IPT_B200_ABI_VERSION; }
@@ -655,17 +697,27 @@ int ipt_device_count(void) {
 }
 
 int ipt_light_derived(const ipt_light* light, float* area, float* surface_power, float normal[3]) {
+    namespace H = ipt_host;
     if (!light) return fail(IPT_ERR_INVALID, "null light");
-    ipt_scene_desc d{};
-    d.n_lights = 1;
-    d.lights = light;
-    std::vector<DevLight> out;
-    float w;
-    int rc = flatten_lights(&d, out, w);
-    if (rc) return rc;
-    if (area) *area = out[0].area;
-    if (surface_power) *surface_power = out[0].surface_power;
-    if (normal) { normal[0] = out[0].nx; normal[1] = out[0].ny; normal[2] = out[0].nz; }
+    const ipt_light& l = *light;
+    float a = 0.0f, sp = NAN; // a point light (lighting.cpp:204)
+    H::f3 nn{0.0f, 0.0f, 0.0f};
+    if (l.kind == IPT_LIGHT_AREA_DIAMOND || l.kind == IPT_LIGHT_AREA_TRIANGLE) {
+        // AreaLight::AreaLight (src/lighting/lighting.cpp:79-90)
+        const H::f3 cr = H::cross(H::mk(l.x_axis), H::mk(l.y_axis));
+        const float full_area = H::length(cr);
+        a = l.kind == IPT_LIGHT_AREA_DIAMOND ? full_area : full_area / 2.0f;
+        nn = H::normalize(cr);
+        sp = l.power / a;
+    } else if (l.kind == IPT_LIGHT_SPHERE || l.kind == IPT_LIGHT_SPHERE_INVERTED) {
+        a = (float)(4.0 * M_PI * l.radius * l.radius); // lighting.h:51
+        sp = l.power / a;
+    } else if (l.kind != IPT_LIGHT_POINT) {
+        return fail(IPT_ERR_INVALID, "unknown light kind");
+    }
+    if (area) *area = a;
+    if (surface_power) *surface_power = sp;
+    if (normal) { normal[0] = nn.x; normal[1] = nn.y; normal[2] = nn.z; }
     return IPT_OK;
 }
 
@@ -683,13 +735,11 @@ int ipt_scene_create(const ipt_scene_desc* desc, int device, ipt_scene** out) {
         if (m.ddf > IPT_DDF_GLOSSY) return fail(IPT_ERR_INVALID, "unknown ddf kind");
     }
     std::vector<DevPrim> prims;
-    std::vector<DevLight> lights;
     bool smallpt = false;
-    float sdf_weight = 1.0f;
     int rc = flatten_prims(desc, prims, smallpt);
     if (rc) return rc;
-    rc = flatten_lights(desc, lights, sdf_weight);
-    if (rc) return rc;
+    for (uint32_t i = 0; i < desc->n_lights; ++i)
+        if (desc->lights[i].kind > IPT_LIGHT_POINT) return fail(IPT_ERR_INVALID, "unknown light kind");
     std::vector<DevMaterial> mats(desc->n_materials);
     for (uint32_t i = 0; i < desc->n_materials; ++i) {
         const ipt_material& m = desc->materials[i];
@@ -726,7 +776,7 @@ int ipt_scene_create(const ipt_scene_desc* desc, int device, ipt_scene** out) {
     dv.n_lights = desc->n_lights;
     dv.n_materials = desc->n_materials;
     dv.has_smallpt = smallpt;
-    dv.sdf_weight = sdf_weight;
+    dv.sdf_weight = desc->n_lights ? 0.5f : 1.0f; // main.cpp:143 unite(light_ddf, 1, sdf, 1); with no lights the sdf alone (ddf.cpp:209-210)
     dv.prim_inline = desc->n_prims <= IPT_INLINE_PRIMS;
     dv.light_inline = desc->n_lights <= IPT_INLINE_LIGHTS;
     bool inline_area_light = dv.light_inline && desc->n_lights > 0; // the lights are the inline ones, all of them area lights
@@ -740,39 +790,10 @@ int ipt_scene_create(const ipt_scene_desc* desc, int device, ipt_scene** out) {
         return e;
     };
     CUDA_TRY(upload(s->d_prims, prims));
-    CUDA_TRY(upload(s->d_lights, lights));
     CUDA_TRY(upload(s->d_mats, mats));
     dv.prims_g = s->d_prims;
-    dv.lights_g = s->d_lights;
-    {
-        std::vector<float> cdf(lights.size());
-        for (size_t i = 0; i < lights.size(); ++i) cdf[i] = lights[i].cdf;
-        CUDA_TRY(upload(s->d_light_cdf, cdf));
-        dv.light_cdf = s->d_light_cdf;
-        // guide[b] = first i with b / M < cdf[i] (DevScene::light_guide); b / M is exact in float
-        std::vector<uint32_t> guide(IPT_LIGHT_GUIDE + 2);
-        size_t i = 0;
-        for (uint32_t b = 0; b <= IPT_LIGHT_GUIDE + 1; ++b) {
-            const float edge = (float)b / (float)IPT_LIGHT_GUIDE;
-            while (i < cdf.size() && !(edge < cdf[i])) ++i;
-            guide[b] = (uint32_t)i;
-        }
-        CUDA_TRY(upload(s->d_light_guide, guide));
-        dv.light_guide = s->d_light_guide;
-        std::vector<float> samp(16 * lights.size());
-        for (size_t k = 0; k < lights.size(); ++k) {
-            const DevLight& L = lights[k];
-            float kind_bits;
-            std::memcpy(&kind_bits, &L.kind, 4);
-            const float rec[16] = {L.px, L.py, L.pz, kind_bits, L.xax, L.xay, L.xaz, L.radius, L.yax, L.yay, L.yaz, 0.0f, L.nx, L.ny, L.nz, 0.0f};
-            std::memcpy(&samp[16 * k], rec, sizeof rec);
-        }
-        CUDA_TRY(upload(s->d_light_samp, samp));
-        dv.light_samp = reinterpret_cast<const float4*>(s->d_light_samp);
-    }
     dv.mats_g = s->d_mats;
     for (uint32_t i = 0; i < desc->n_prims && i < IPT_INLINE_PRIMS; ++i) dv.prims[i] = prims[i];
-    for (uint32_t i = 0; i < desc->n_lights && i < IPT_INLINE_LIGHTS; ++i) dv.lights[i] = lights[i];
     for (uint32_t i = 0; i < desc->n_materials && i < IPT_INLINE_MATS; ++i) dv.mats[i] = mats[i];
     // group the box planes by (axis, sign) for the branch-free plane test
     dv.planes_grouped = 1;
@@ -798,41 +819,27 @@ int ipt_scene_create(const ipt_scene_desc* desc, int device, ipt_scene** out) {
     s->mesh = desc->n_triangles > 0;
     // grouped box planes + inline spheres only (analytic_closest's first branch)
     const bool geom_fast = geom_fast_scene(s);
-    dv.lights_inside_box = lights_inside_box(dv, geom_fast && inline_area_light, desc->lights, desc->n_lights);
     bool all_lambert = true; // every material is the cosine DDF
     for (const DevMaterial& m : mats) if (m.ddf != IPT_DDF_COSINE) all_lambert = false;
     if (s->mesh) {
+        DevBuf<float> staged;
+        const float* d_tris;
+        CUDA_TRY(stage_input(s, desc->triangles, 9 * (size_t)desc->n_triangles, false, staged, &d_tris));
         std::string err;
-        if (lbvh_build_host(desc->triangles, (uint32_t)desc->n_triangles, s->stream, s->bvh, err) != 0)
-            return fail(IPT_ERR_CUDA, "LBVH build failed: " + err);
+        if (lbvh_build(d_tris, (uint32_t)desc->n_triangles, s->stream, s->bvh, err) != 0) return fail(IPT_ERR_CUDA, "LBVH build failed: " + err);
         dv.n_tris = (uint32_t)desc->n_triangles;
         dv.tri_material = desc->triangle_material;
         bind_mesh(s);
     }
     // many area lights: LBVH over them (nearest-light and all-hits density queries instead of O(L) scans)
+    bool all_area = desc->n_lights > 0;
+    for (uint32_t i = 0; i < desc->n_lights; ++i) all_area = all_area && desc->lights[i].kind <= IPT_LIGHT_AREA_TRIANGLE;
+    if (all_area && desc->n_lights > IPT_LIGHT_BVH_MIN) dv.n_light_bvh = desc->n_lights;
     {
-        bool all_area = desc->n_lights > 0;
-        for (uint32_t i = 0; i < desc->n_lights; ++i) all_area = all_area && desc->lights[i].kind <= IPT_LIGHT_AREA_TRIANGLE;
-        if (all_area && desc->n_lights > IPT_LIGHT_BVH_MIN) {
-            std::vector<float> ltris(9 * (size_t)desc->n_lights), extra(3 * (size_t)desc->n_lights);
-            for (uint32_t i = 0; i < desc->n_lights; ++i) {
-                const ipt_light& l = desc->lights[i];
-                std::memcpy(&ltris[9 * (size_t)i], l.position, 12);
-                std::memcpy(&ltris[9 * (size_t)i + 3], l.x_axis, 12);
-                std::memcpy(&ltris[9 * (size_t)i + 6], l.y_axis, 12);
-                extra[3 * (size_t)i] = l.kind == IPT_LIGHT_AREA_TRIANGLE ? 1.0f : 0.0f;
-                extra[3 * (size_t)i + 1] = lights[i].area;
-                extra[3 * (size_t)i + 2] = lights[i].weight;
-            }
-            std::string err;
-            if (lbvh_build_host(ltris.data(), desc->n_lights, s->stream, s->light_bvh, err, extra.data()) != 0)
-                return fail(IPT_ERR_CUDA, "light LBVH build failed: " + err);
-            dv.light_nodes = s->light_bvh.nodes;
-            dv.light_qnodes = s->light_bvh.qnodes;
-            dv.light_grid = s->light_bvh.grid;
-            dv.light_recs = s->light_bvh.tri_records;
-            dv.n_light_bvh = desc->n_lights;
-        }
+        DevBuf<ipt_light> staged;
+        const ipt_light* d_in;
+        CUDA_TRY(stage_input(s, desc->lights, desc->n_lights, false, staged, &d_in));
+        if (int rc = derive_lights(s, d_in, desc->n_lights, true, "")) return rc;
     }
     CUDA_TRY(cudaMalloc((void**)&s->d_cnt, sizeof(uint32_t) * IPT_CNT_WORDS));
     CUDA_TRY(cudaMalloc((void**)&s->d_stats, sizeof(unsigned long long) * ST_COUNT));
@@ -933,12 +940,8 @@ int ipt_scene_update_triangles(ipt_scene* s, const float* triangles, uint64_t n_
     if (int rc = check_input_pointer(s, triangles, device_input, alignof(float), "ipt_scene_update_triangles", "triangles", "a float")) return rc;
     const uint32_t n = s->bvh.n;
     DevBuf<float> staged;
-    const float* d_tris = triangles;
-    if (!device_input) { // the copy lbvh_build_host makes at scene creation
-        CUDA_TRY(staged.alloc(9 * (size_t)n));
-        CUDA_TRY(cudaMemcpyAsync(staged.p, triangles, sizeof(float) * 9 * (size_t)n, cudaMemcpyHostToDevice, s->stream));
-        d_tris = staged.p;
-    }
+    const float* d_tris;
+    CUDA_TRY(stage_input(s, triangles, 9 * (size_t)n, device_input, staged, &d_tris));
     std::string err;
     if (flags & IPT_UPDATE_REBUILD) {
         // into a new tree: the scene keeps the old one unless the build succeeds. lbvh_build waits for the scene stream, so
@@ -1027,95 +1030,11 @@ int ipt_scene_update_lights(ipt_scene* s, const ipt_light* lights, uint32_t n_li
     CUDA_TRY(cudaSetDevice(s->device));
     const bool device_input = flags & IPT_UPDATE_DEVICE_POINTER;
     if (int rc = check_input_pointer(s, lights, device_input, alignof(uint32_t), entry, "lights", "4 bytes")) return rc;
-    const uint32_t n = n_lights;
-    if (n == 0) return IPT_OK;
-    const bool tree = dv.n_light_bvh > 0;
-    // new buffers, filled and checked before anything of the scene changes
+    if (n_lights == 0) return IPT_OK;
     DevBuf<ipt_light> staged;
-    DevBuf<DevLight> d_lights;
-    DevBuf<float> cdf, samp, scratch, ltris, extra;
-    DevBuf<uint32_t> guide, word;
-    CUDA_TRY(d_lights.alloc(n));
-    CUDA_TRY(cdf.alloc(n));
-    CUDA_TRY(samp.alloc(16 * (size_t)n));
-    CUDA_TRY(scratch.alloc(4 * (size_t)n)); // ka, f, r, w
-    CUDA_TRY(guide.alloc(IPT_LIGHT_GUIDE + 2));
-    CUDA_TRY(word.alloc(1));
-    if (tree) {
-        CUDA_TRY(ltris.alloc(9 * (size_t)n));
-        CUDA_TRY(extra.alloc(3 * (size_t)n));
-    }
-    const ipt_light* d_in = lights;
-    if (!device_input) {
-        CUDA_TRY(staged.alloc(n));
-        CUDA_TRY(cudaMemcpyAsync(staged.p, lights, sizeof(ipt_light) * (size_t)n, cudaMemcpyHostToDevice, s->stream));
-        d_in = staged.p;
-    }
-    float *ka = scratch.p, *f = ka + n, *r = f + n, *w = r + n;
-    const unsigned blocks = (n + 255) / 256;
-    CUDA_TRY(cudaMemsetAsync(word.p, 0xFF, sizeof(uint32_t), s->stream));
-    k_light_derive<<<blocks, 256, 0, s->stream>>>(d_in, n, s->d_lights, d_lights.p, reinterpret_cast<float4*>(samp.p), ltris.p, extra.p, word.p);
-    k_light_power_prefix<<<1, 1, 0, s->stream>>>(d_in, n, ka);
-    k_light_ratios<<<blocks, 256, 0, s->stream>>>(d_in, ka, n, f, r);
-    const uint32_t weight_threads = (n + IPT_WEIGHTS_PER_THREAD - 1) / IPT_WEIGHTS_PER_THREAD;
-    k_light_weights<<<(weight_threads + 127) / 128, 128, 0, s->stream>>>(f, r, n, w, d_lights.p, extra.p);
-    k_light_scan<<<1, 1, 0, s->stream>>>(w, n, cdf.p, d_lights.p, guide.p);
-    CUDA_TRY(cudaGetLastError());
-    // what the host needs back: the kind check and, for a scene that holds its light inline, the derived record and the
-    // input record (DevScene::lights and lights_inside_box)
-    uint32_t first_bad = 0;
-    DevLight inline_derived[IPT_INLINE_LIGHTS];
-    ipt_light inline_input[IPT_INLINE_LIGHTS];
-    const uint32_t n_inline = dv.light_inline ? n : 0; // n <= IPT_INLINE_LIGHTS
-    CUDA_TRY(cudaMemcpyAsync(&first_bad, word.p, sizeof first_bad, cudaMemcpyDeviceToHost, s->stream));
-    if (n_inline) {
-        CUDA_TRY(cudaMemcpyAsync(inline_derived, d_lights.p, sizeof(DevLight) * n_inline, cudaMemcpyDeviceToHost, s->stream));
-        CUDA_TRY(cudaMemcpyAsync(inline_input, d_in, sizeof(ipt_light) * n_inline, cudaMemcpyDeviceToHost, s->stream));
-    }
-    CUDA_TRY(cudaStreamSynchronize(s->stream));
-    if (first_bad != 0xFFFFFFFFu)
-        return fail(IPT_ERR_INVALID, std::string(entry) + ": lights[" + std::to_string(first_bad) + "].kind differs from the kind of the scene's light " +
-                                         std::to_string(first_bad) + " (a different kind needs a new scene)");
-    // the light LBVH: a rebuild goes into a new tree, swapped in only if the build succeeds; a refit allocates all its scratch
-    // before it writes the tree
-    LbvhDevice fresh;
-    bool rebuilt = false;
-    if (tree) {
-        std::string err;
-        if (flags & IPT_UPDATE_REBUILD) {
-            if (lbvh_build(ltris.p, n, s->stream, fresh, err, extra.p) != 0) return fail(IPT_ERR_CUDA, std::string(entry) + ": light LBVH build failed: " + err);
-            rebuilt = true;
-        } else if (lbvh_refit(ltris.p, s->stream, s->light_bvh, err, extra.p) != 0) {
-            return fail(IPT_ERR_CUDA, std::string(entry) + ": light LBVH refit failed: " + err);
-        }
-    }
-    // commit. The stream is idle (the tree stages end with a synchronise): no enqueued render still reads the buffers that
-    // are replaced, and the DevBufs free them on return.
-    std::swap(s->d_lights, d_lights.p);
-    std::swap(s->d_light_cdf, cdf.p);
-    std::swap(s->d_light_guide, guide.p);
-    std::swap(s->d_light_samp, samp.p);
-    dv.lights_g = s->d_lights;
-    dv.light_cdf = s->d_light_cdf;
-    dv.light_guide = s->d_light_guide;
-    dv.light_samp = reinterpret_cast<const float4*>(s->d_light_samp);
-    if (rebuilt) {
-        lbvh_free(s->light_bvh);
-        s->light_bvh = fresh;
-    }
-    if (tree) {
-        dv.light_nodes = s->light_bvh.nodes;
-        dv.light_qnodes = s->light_bvh.qnodes;
-        dv.light_grid = s->light_bvh.grid;
-        dv.light_recs = s->light_bvh.tri_records;
-    }
-    bool inline_area_light = n_inline > 0;
-    for (uint32_t i = 0; i < n_inline; ++i) {
-        dv.lights[i] = inline_derived[i];
-        if (inline_input[i].kind > IPT_LIGHT_AREA_TRIANGLE) inline_area_light = false;
-    }
-    dv.lights_inside_box = lights_inside_box(dv, geom_fast_scene(s) && inline_area_light, inline_input, n_inline);
-    return IPT_OK;
+    const ipt_light* d_in;
+    CUDA_TRY(stage_input(s, lights, n_lights, device_input, staged, &d_in));
+    return derive_lights(s, d_in, n_lights, flags & IPT_UPDATE_REBUILD, std::string(entry) + ": ");
 }
 
 // ---- parity entries ----------------------------------------------------------------------------------
@@ -1308,6 +1227,28 @@ int ipt_bvh_export_compact(ipt_scene* s, uint32_t* nodes32, float grid[6], uint6
     if (n_nodes) *n_nodes = n > 1 ? n - 1 : 0;
     if (nodes32 && n > 1) CUDA_TRY(cudaMemcpy(nodes32, s->bvh.qnodes, sizeof(BvhNodeQ) * (size_t)(n - 1), cudaMemcpyDeviceToHost));
     if (grid) for (int a = 0; a < 3; ++a) { grid[a] = s->bvh.grid.lo[a]; grid[3 + a] = s->bvh.grid.scale[a]; }
+    return IPT_OK;
+}
+
+int ipt_light_tables_export(ipt_scene* s, float* area, float* surface_power, float* normal, float* weight, float* cdf,
+                            uint32_t guide[IPT_LIGHT_GUIDE_WORDS]) {
+    static_assert(IPT_LIGHT_GUIDE_WORDS == IPT_LIGHT_GUIDE + 2, "ABI guide size");
+    if (!s) return fail(IPT_ERR_INVALID, "null scene");
+    std::lock_guard<std::recursive_mutex> lock__(s->mu);
+    CUDA_TRY(cudaSetDevice(s->device));
+    CUDA_TRY(cudaStreamSynchronize(s->stream));
+    const uint32_t n = s->dev.n_lights;
+    std::vector<DevLight> lights(n);
+    if (n) CUDA_TRY(cudaMemcpy(lights.data(), s->d_lights, sizeof(DevLight) * n, cudaMemcpyDeviceToHost));
+    for (uint32_t i = 0; i < n; ++i) {
+        const DevLight& L = lights[i];
+        if (area) area[i] = L.area;
+        if (surface_power) surface_power[i] = L.surface_power;
+        if (normal) { normal[3 * i] = L.nx; normal[3 * i + 1] = L.ny; normal[3 * i + 2] = L.nz; }
+        if (weight) weight[i] = L.weight;
+    }
+    if (cdf && n) CUDA_TRY(cudaMemcpy(cdf, s->d_light_cdf, sizeof(float) * n, cudaMemcpyDeviceToHost));
+    if (guide) CUDA_TRY(cudaMemcpy(guide, s->d_light_guide, sizeof(uint32_t) * IPT_LIGHT_GUIDE_WORDS, cudaMemcpyDeviceToHost));
     return IPT_OK;
 }
 

@@ -426,25 +426,6 @@ fail:
     return 1;
 }
 
-// The same from HOST memory: the triangles (and extras) are staged on the stream, then built.
-static inline int lbvh_build_host(const float* host_tris, uint32_t n, cudaStream_t st, LbvhDevice& out, std::string& err,
-                                  const float* host_extra = nullptr) {
-    float* d_tris = nullptr;
-    float* d_extra = nullptr;
-    int rc = 1;
-    out = LbvhDevice();
-    LB_TRY(cudaMalloc((void**)&d_tris, sizeof(float) * 9 * (size_t)n));
-    LB_TRY(cudaMemcpyAsync(d_tris, host_tris, sizeof(float) * 9 * (size_t)n, cudaMemcpyHostToDevice, st));
-    if (host_extra) {
-        LB_TRY(cudaMalloc((void**)&d_extra, sizeof(float) * 3 * (size_t)n));
-        LB_TRY(cudaMemcpyAsync(d_extra, host_extra, sizeof(float) * 3 * (size_t)n, cudaMemcpyHostToDevice, st));
-    }
-    rc = lbvh_build(d_tris, n, st, out, err, d_extra);
-fail:
-    cudaFree(d_extra); cudaFree(d_tris);
-    return rc;
-}
-
 // Refit: new vertices (DEVICE memory, the triangle count of the tree) under the tree's kept topology and sorted order.
 // Recomputes the leaf boxes, the internal boxes, the records, the grid and the 32-byte nodes in place; the Morton keys and
 // sorted order stay those of the build. All scratch is allocated before anything of `b` is written: on an allocation

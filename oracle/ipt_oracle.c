@@ -913,6 +913,25 @@ int ipt_oracle_light_fields(const ipt_scene_desc* desc, uint32_t i, float* out5)
     return 0;
 }
 
+/* the light tables a scene's lights make: per light prepare_light's area, surface power and normal (3 floats) and
+ * prepare_weights' mixture weight */
+int ipt_oracle_light_tables(const ipt_scene_desc* desc, float* area, float* surface_power, float* normal, float* weight) {
+    oscene s;
+    memset(&s, 0, sizeof s);
+    s.d = desc;
+    prepare_weights(&s);
+    for (uint32_t i = 0; i < desc->n_lights; ++i) {
+        olight L;
+        prepare_light(&L, &desc->lights[i]);
+        area[i] = L.area;
+        surface_power[i] = L.surface_power;
+        normal[3 * i] = L.normal.x; normal[3 * i + 1] = L.normal.y; normal[3 * i + 2] = L.normal.z;
+        weight[i] = s.light_w[i];
+    }
+    free(s.light_w);
+    return 0;
+}
+
 /* Philox known-answer access for tests */
 void ipt_oracle_philox_rounds(int rounds, uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1, uint32_t* out) {
     philox4x32_r(rounds, c0, c1, c2, c3, k0, k1, out);

@@ -211,6 +211,13 @@ class Oracle(_OutputStage):
         self.lib.ipt_oracle_light_fields(desc_ptr, C.c_uint32(i), _p(out, f32p))
         return out
 
+    def light_tables(self, desc_ptr, n_lights):
+        """Per light the area, surface power, normal (n, 3) and mixture weight the oracle derives, as float32 arrays."""
+        area, sp, w = (np.empty(n_lights, np.float32) for _ in range(3))
+        normal = np.empty((n_lights, 3), np.float32)
+        assert self.lib.ipt_oracle_light_tables(desc_ptr, _p(area, f32p), _p(sp, f32p), _p(normal, f32p), _p(w, f32p)) == 0
+        return dict(area=area, surface_power=sp, normal=normal, weight=w)
+
     def bvh_build(self, triangles):
         """The LBVH exactly as ipt_b200/csrc/ipt_lbvh.cuh builds it: (nodes, sorted ids, sorted Morton keys)."""
         from ipt_b200.capi import BVH_NODE_DTYPE

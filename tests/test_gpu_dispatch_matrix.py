@@ -548,7 +548,8 @@ def test_l3_produces_exactly_tied_nearest_lights(lib, oracle):
 
 
 def _cdf(power):
-    """The light part of the mixture cdf as flatten_lights (ipt_capi.cu) builds it, in float32."""
+    """The light part of the mixture cdf as the device derivation (k_light_weights and k_light_scan, ipt_capi.cu) builds
+    it, in float32."""
     n = len(power)
     w = np.zeros(n, np.float32)
     acc = np.float32(0)

@@ -1,5 +1,6 @@
-"""GPU checks of ipt_scene_update_lights (Scene.update_lights): the light tables, the light LBVH and lights_inside_box
-derived on the device equal what ipt_scene_create derives on the host. Updating a scene with its own lights changes
+"""GPU checks of ipt_scene_update_lights (Scene.update_lights): the light tables, the light LBVH and lights_inside_box of
+an updated scene equal those of a scene created with the new lights (test_gpu_light_tables.py compares the tables of both
+with the oracle). Updating a scene with its own lights changes
 nothing; after moving and re-powering the lights, a rebuilt scene equals a fresh scene of the new lights bit for bit, and a
 refitted one equals it except for the light tree's traversal counters and the summation order of the all-hits density. The light
 sets and rays are those of test_gpu_dispatch_matrix.py; every case runs for host and device input and for refit and
